@@ -16,6 +16,7 @@ independent, every rank works on its own shard, no data-path collective -- SURVE
              job through ONE process whose DASContext spans the N devices (EKZG_DEVICES), the way a binding would use the box.
   configs  : (N = 1) BASELINE configs #1, #2, #4, #5 at full size with >= 64 items each checked against the CPU oracle;
   abi_single_blob : (N = 1) tools/abi_load.c, 1024 native threads calling the reference's per-blob symbol.
+  --dump-outputs DIR : what the timed path (either arm) returned in its last step, as .npy files (see dump_outputs).
 Prints ONE JSON line on rank 0."""
 import argparse
 import ctypes
@@ -26,6 +27,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as the build left it (which may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -46,6 +48,8 @@ OP_JAC_DBL = 2 * IMAD_MUL + 5 * IMAD_SQR
 OP_JAC_MADD = 7 * IMAD_MUL + 4 * IMAD_SQR
 OP_JAC_ADD = 11 * IMAD_MUL + 5 * IMAD_SQR
 OP_MADD_ZR = 8 * IMAD_MUL + 3 * IMAD_SQR
+DUMP_BYTES = 64 * 10**6             # --dump-outputs: all files together, .npy headers included
+DUMP_SEED = 0xB200
 
 
 def k5_imad_per_blob():
@@ -148,6 +152,30 @@ def workload_config(n):
             "sharding": "independent blobs per rank, tables replicated, no collective"}
 
 
+def dump_outputs(out_dir, n, d_cells, d_proofs, d_status):
+    """What one step of the timed path returned for n blobs, one float32 per output byte (exact: bytes are 0..255),
+    so that two builds (or the two arms) can be compared file for file on the same synthetic inputs:
+      status.npy [n]                      per-blob status (0 = ok)
+      proofs.npy [k, 128, 48]             compressed G1 proofs
+      cells.npy [k', 128, 2048]           cells
+      proofs_blobs.npy, cells_blobs.npy   which blobs (float64 indices): all n, or a fixed seeded sample (sorted) where the
+                                          whole output would not fit in DUMP_BYTES; proofs get up to half of it"""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    status = d_status.to(torch.float32).cpu().numpy()
+    left = DUMP_BYTES - status.nbytes - 5 * 128               # 128: one .npy header
+    for name, rows, share in (("proofs", d_proofs.view(n, 128, 48), 0.5), ("cells", d_cells.view(n, 128, 2048), 1.0)):
+        per_blob = 4 * rows[0].numel() + 8                     # its float32 values and its float64 index
+        k = min(n, int(left * share) // per_blob)
+        idx = np.arange(n) if k == n else np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+        out = rows[torch.from_numpy(idx).to(rows.device)].to(torch.float32).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), out)
+        np.save(os.path.join(out_dir, name + "_blobs.npy"), idx.astype(np.float64))
+        left -= out.nbytes + 8 * k
+    np.save(os.path.join(out_dir, "status.npy"), status)
+
+
 def port_note():
     return ("C restatement of the reference algorithm (oracle/, 64-bit limbs + __int128, no assembly); the Rust/blst reference cannot be built in this "
             "image (no cargo).  fp_mul_ns is this port's measured Montgomery multiplication on one core of this box; blst's assembly is ~25-30 ns "
@@ -192,8 +220,12 @@ def run_reference(args, rank, world):
         cref.compute_cells_and_kzg_proofs_batch(blobs, per_step, cores)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cref.compute_cells_and_kzg_proofs_batch(blobs, per_step, cores)
+        out = cref.compute_cells_and_kzg_proofs_batch(blobs, per_step, cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        import torch
+        cells, proofs = (torch.frombuffer(bytearray(b), dtype=torch.uint8) for b in out)
+        dump_outputs(args.dump_outputs, per_step, cells, proofs, torch.zeros(per_step, dtype=torch.int32))
     v = per_step * args.steps / dt
     cfg = workload_config(n)
     if per_step != n:
@@ -308,7 +340,10 @@ def main():
     ap.add_argument("--precomp", type=int, default=1, help="use_precomp flag of the context (window from EKZG_FK20_WINDOW)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline only: skip configs / latency / abi_single_blob / one-process multi-device")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0's blobs) to DIR/*.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -400,6 +435,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     # parity spot check inside the bench: device-resident and host paths agree
     assert torch.equal(h_proofs.cuda(), d_proofs) and torch.equal(h_cells.cuda(), d_cells), "device and host paths disagree"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, n, d_cells, d_proofs, d_status)
 
     t = torch.tensor([dev_ms, e2e_ms], dtype=torch.float64, device="cuda")
     if world > 1:
