@@ -40,6 +40,34 @@ static const ekzg::DeviceSet& ds(const DASContext* ctx) {
 static const ekzg::Context& cx(const DASContext* ctx) { return ds(ctx).primary(); }      // calls that use one device
 static const ekzg::Context& next_cx(const DASContext* ctx) { return ds(ctx).next(); }    // single-item calls: round-robin
 
+// The two stage hooks: one blob through K1, K2 and K4 (the kernels without scratch) on a borrowed workspace's stream, then
+// tail(ws, stream), which returns its failing step or nullptr.  Synchronous.
+template <class Tail>
+static CResult debug_fk20_run(const DASContext* ctx, const uint8_t* blob, Tail tail) {
+    using namespace ekzg;
+    DeviceGuard guard;
+    const Context& c = cx(ctx);
+    Status s = c.bind_device();
+    if (!s.ok) return c_err(s.msg);
+    Workspace* ws = c.acquire(1, true);
+    if (!ws) return c_err("allocation failed");
+    cudaStream_t st = ws->stream;
+    const DevTables& T = c.tables();
+    auto run = [&]() -> const char* {
+        if (cudaMemcpyAsync(ws->d_blobs, blob, BYTES_PER_BLOB, cudaMemcpyHostToDevice, st) != cudaSuccess) return "h2d";
+        cudaMemsetAsync(ws->d_status, 0, 4, st);
+        if (launch_blob_to_coeffs_cells(ws->d_blobs, ws->d_coeffs, ws->d_cells, ws->d_status, T, 1, true, st) != cudaSuccess) return "k1";
+        if (launch_toeplitz_scalars(ws->d_coeffs, ws->d_scalars, T, 1, st) != cudaSuccess) return "k2";
+        if (launch_fixed_msm(ws->d_scalars, ws->d_pts, T.fk20, FK20_MSMS, 1, st) != cudaSuccess) return "k4";
+        if (const char* m = tail(*ws, st)) return m;
+        const cudaError_t e = cudaStreamSynchronize(st);
+        return e == cudaSuccess ? nullptr : cudaGetErrorString(e);
+    };
+    const char* m = run();
+    c.give_back(ws, m ? Status::Error(m) : Status::Ok());
+    return m ? c_err(m) : c_ok();
+}
+
 extern "C" {
 
 DASContext* eth_kzg_das_context_new(bool use_precomp) {
@@ -132,8 +160,7 @@ CResult eth_kzg_b200_compute_cells_and_kzg_proofs_device(const DASContext* ctx, 
     const ekzg::Context& c = *owner;
     Status s = c.bind_device();
     if (!s.ok) return c_err(s.msg);
-    // (one or two blobs take the direct proof path, which wants room for 128 virtual blobs per blob: kzg_runtime.h)
-    ekzg::Workspace* ws = c.acquire(d_proofs && n <= (uint64_t)ekzg::direct_proofs_max() ? ekzg::N_CELLS * (int)n : (int)n, false);
+    ekzg::Workspace* ws = c.acquire(ekzg::proof_route(n, (int)n, d_proofs != nullptr).capacity, false);
     if (!ws) return c_err("device memory allocation failed");
     cudaStream_t st = (cudaStream_t)cuda_stream;
     cudaStreamWaitEvent(st, ws->done, 0);  // the scratch buffers' previous user may have run on another stream
@@ -143,7 +170,7 @@ CResult eth_kzg_b200_compute_cells_and_kzg_proofs_device(const DASContext* ctx, 
     cudaEventRecord(ws->done, st);
     cudaStreamWaitEvent(ws->stream, ws->done, 0);
     if (!s.ok) cudaGetLastError();
-    c.give_back(ws);
+    c.give_back(ws, s);
     return to_c(s);
 }
 
@@ -178,31 +205,19 @@ int eth_kzg_b200_collect_stage_times(const DASContext* ctx, double* ms_out) {
 // MSM outputs (natural j order) and h commitments as compressed points.  Synchronous; test hook.
 CResult eth_kzg_b200_debug_fk20_stages(const DASContext* ctx, const uint8_t* blob, uint32_t* out_scalars, uint8_t* out_msm, uint8_t* out_h) {
     using namespace ekzg;
-    DeviceGuard guard;
-    const Context& c = cx(ctx);
-    Status s = c.bind_device();
-    if (!s.ok) return c_err(s.msg);
-    Workspace* ws = c.acquire(1, true);
-    if (!ws) return c_err("allocation failed");
-    cudaStream_t st = ws->stream;
-    const DevTables& T = c.tables();
-    auto fail = [&](const char* m) { c.give_back(ws); return c_err(m); };
-    if (cudaMemcpyAsync(ws->d_blobs, blob, BYTES_PER_BLOB, cudaMemcpyHostToDevice, st) != cudaSuccess) return fail("h2d");
-    cudaMemsetAsync(ws->d_status, 0, 4, st);
-    if (launch_blob_to_coeffs_cells(ws->d_blobs, ws->d_coeffs, ws->d_cells, ws->d_status, T, 1, true, st) != cudaSuccess) return fail("k1");
-    if (launch_toeplitz_scalars(ws->d_coeffs, ws->d_scalars, T, 1, st) != cudaSuccess) return fail("k2");
-    if (cudaMemcpyAsync(out_scalars, ws->d_scalars, 128 * 64 * 32, cudaMemcpyDeviceToHost, st) != cudaSuccess) return fail("d2h scalars");
-    if (launch_fixed_msm(ws->d_scalars, ws->d_pts, T.fk20, FK20_MSMS, 1, st) != cudaSuccess) return fail("k4");
-    // MSM outputs sit at bit-reversed positions; compress all 128 then un-permute on the host
-    if (launch_g1_compress(ws->d_pts, ws->d_proofs, 128, 1, st) != cudaSuccess) return fail("k6");
     uint8_t tmp[128 * 48];
-    if (cudaMemcpyAsync(tmp, ws->d_proofs, sizeof(tmp), cudaMemcpyDeviceToHost, st) != cudaSuccess) return fail("d2h msm");
-    if (launch_g1_ntt_phases(ws->d_pts, 1, 0, 7, ws->d_queue, ws->d_ntt_scratch, st) != cudaSuccess) return fail("k5");
-    if (launch_g1_compress(ws->d_pts, ws->d_proofs, 64, 1, st) != cudaSuccess) return fail("k6b");
-    if (cudaMemcpyAsync(out_h, ws->d_proofs, 64 * 48, cudaMemcpyDeviceToHost, st) != cudaSuccess) return fail("d2h h");
-    cudaError_t e = cudaStreamSynchronize(st);
-    c.give_back(ws);
-    if (e != cudaSuccess) return c_err(cudaGetErrorString(e));
+    CResult res = debug_fk20_run(ctx, blob, [&](Workspace& ws, cudaStream_t st) -> const char* {
+        // (K4 leaves the scalars as they are)
+        if (cudaMemcpyAsync(out_scalars, ws.d_scalars, 128 * 64 * 32, cudaMemcpyDeviceToHost, st) != cudaSuccess) return "d2h scalars";
+        // MSM outputs sit at bit-reversed positions; compress all 128 then un-permute on the host
+        if (launch_g1_compress(ws.d_pts, ws.d_proofs, 128, 1, st) != cudaSuccess) return "k6";
+        if (cudaMemcpyAsync(tmp, ws.d_proofs, sizeof(tmp), cudaMemcpyDeviceToHost, st) != cudaSuccess) return "d2h msm";
+        if (launch_g1_ntt_phases(ws.d_pts, 1, 0, 7, ws.d_queue, ws.d_ntt_scratch, st) != cudaSuccess) return "k5";
+        if (launch_g1_compress(ws.d_pts, ws.d_proofs, 64, 1, st) != cudaSuccess) return "k6b";
+        if (cudaMemcpyAsync(out_h, ws.d_proofs, 64 * 48, cudaMemcpyDeviceToHost, st) != cudaSuccess) return "d2h h";
+        return nullptr;
+    });
+    if (res.status != Ok) return res;
     for (int j = 0; j < 128; j++) {
         int r = 0;
         for (int b = 0; b < 7; b++) r |= ((j >> b) & 1) << (6 - b);
@@ -215,28 +230,13 @@ CResult eth_kzg_b200_debug_fk20_stages(const DASContext* ctx, const uint8_t* blo
 // in storage order.  With EKZG_K5_R4_MAX >= 1 and an even `phases` the radix-4 kernel runs its first phases / 2 super-phases.
 CResult eth_kzg_b200_debug_g1_ntt_prefix(const DASContext* ctx, const uint8_t* blob, int phases, uint8_t* out128x48) {
     using namespace ekzg;
-    DeviceGuard guard;
-    const Context& c = cx(ctx);
-    Status s = c.bind_device();
-    if (!s.ok) return c_err(s.msg);
     if (phases < 0 || phases > 14) return c_err("phases out of range");
-    Workspace* ws = c.acquire(1, true);
-    if (!ws) return c_err("allocation failed");
-    cudaStream_t st = ws->stream;
-    const DevTables& T = c.tables();
-    auto fail = [&](const char* m) { c.give_back(ws); return c_err(m); };
-    if (cudaMemcpyAsync(ws->d_blobs, blob, BYTES_PER_BLOB, cudaMemcpyHostToDevice, st) != cudaSuccess) return fail("h2d");
-    cudaMemsetAsync(ws->d_status, 0, 4, st);
-    if (launch_blob_to_coeffs_cells(ws->d_blobs, ws->d_coeffs, ws->d_cells, ws->d_status, T, 1, true, st) != cudaSuccess) return fail("k1");
-    if (launch_toeplitz_scalars(ws->d_coeffs, ws->d_scalars, T, 1, st) != cudaSuccess) return fail("k2");
-    if (launch_fixed_msm(ws->d_scalars, ws->d_pts, T.fk20, FK20_MSMS, 1, st) != cudaSuccess) return fail("k4");
-    if (phases > 0 && launch_g1_ntt_phases(ws->d_pts, 1, 0, phases, ws->d_queue, ws->d_ntt_scratch, st) != cudaSuccess) return fail("k5");
-    if (launch_g1_compress(ws->d_pts, ws->d_proofs, 128, 1, st) != cudaSuccess) return fail("k6");
-    if (cudaMemcpyAsync(out128x48, ws->d_proofs, 128 * 48, cudaMemcpyDeviceToHost, st) != cudaSuccess) return fail("d2h");
-    cudaError_t e = cudaStreamSynchronize(st);
-    c.give_back(ws);
-    if (e != cudaSuccess) return c_err(cudaGetErrorString(e));
-    return c_ok();
+    return debug_fk20_run(ctx, blob, [&](Workspace& ws, cudaStream_t st) -> const char* {
+        if (phases > 0 && launch_g1_ntt_phases(ws.d_pts, 1, 0, phases, ws.d_queue, ws.d_ntt_scratch, st) != cudaSuccess) return "k5";
+        if (launch_g1_compress(ws.d_pts, ws.d_proofs, 128, 1, st) != cudaSuccess) return "k6";
+        if (cudaMemcpyAsync(out128x48, ws.d_proofs, 128 * 48, cudaMemcpyDeviceToHost, st) != cudaSuccess) return "d2h";
+        return nullptr;
+    });
 }
 
 // Test hook (host only, needs no GPU): prod e(P_i, Q_i) == 1 for affine G1 points given as 96 bytes each (x then y, plain

@@ -13,6 +13,8 @@ constexpr int N_CELLS = 128;         // CELLS_PER_EXT_BLOB
 constexpr int BYTES_PER_BLOB = 131072;
 constexpr int BYTES_PER_CELL = 2048;
 constexpr int BYTES_PER_G1 = 48;
+constexpr size_t CELLS_PER_BLOB = (size_t)N_EXT * 32;              // bytes of the 128 cells of a blob
+constexpr size_t PROOFS_PER_BLOB = (size_t)N_CELLS * BYTES_PER_G1; // bytes of its 128 proofs
 constexpr int FK20_POINTS = 64;      // points per fixed-base MSM  (fk20/prover.rs:95-104)
 constexpr int FK20_MSMS = 128;       // MSMs per blob = circulant domain size (fk20/batch_toeplitz.rs:113)
 

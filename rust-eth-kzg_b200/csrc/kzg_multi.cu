@@ -113,7 +113,6 @@ Status DeviceSet::fan_out(uint64_t n, const std::function<Status(const Context&,
 
 Status DeviceSet::compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* blobs, uint8_t* cells, uint8_t* proofs, uint8_t* blob_status,
                                                      bool want_proofs) const {
-    constexpr size_t CELLS_PER_BLOB = (size_t)N_EXT * 32, PROOFS_PER_BLOB = (size_t)N_CELLS * BYTES_PER_G1;
     return fan_out(n, [&](const Context& c, uint64_t lo, uint64_t cnt) {
         return c.compute_cells_and_kzg_proofs_batch(cnt, blobs + lo * BYTES_PER_BLOB, cells ? cells + lo * CELLS_PER_BLOB : nullptr,
                                                     proofs ? proofs + lo * PROOFS_PER_BLOB : nullptr, blob_status ? blob_status + lo : nullptr, want_proofs);
@@ -137,7 +136,6 @@ Status DeviceSet::compute_blob_kzg_proof_batch(uint64_t n, const uint8_t* blobs,
 Status DeviceSet::recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
                                                      uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const {
     if (ctx_.size() == 1 || n <= 8) return ctx_[0]->recover_cells_and_kzg_proofs_batch(n, counts, indices, cells, out_cells, out_proofs, item_status);
-    constexpr size_t CELLS_PER_BLOB = (size_t)N_EXT * 32, PROOFS_PER_BLOB = (size_t)N_CELLS * BYTES_PER_G1;
     std::vector<uint64_t> offset(n + 1, 0);   // blob i's cells and indices start at offset[i] in the concatenated inputs
     for (uint64_t i = 0; i < n; i++) offset[i + 1] = offset[i] + counts[i];
     return fan_out(n, [&](const Context& c, uint64_t lo, uint64_t cnt) {

@@ -69,10 +69,24 @@ void host_blob_challenge(const uint8_t* blob, const uint8_t* commitment48, uint8
         for (int b = 0; b < 8; b++) z_be[8 * (3 - i) + b] = (uint8_t)(v[i] >> (8 * (7 - b)));
 }
 
-int direct_proofs_max() {
+static int direct_proofs_max() {
     const char* e = getenv("EKZG_DIRECT_MAX");
     const int v = e ? atoi(e) : 1;   // two blobs: 8.2 ms direct against 7.0 ms through FK20 with the cooperative G1 NTTs (profiles/r2_latency_sweep.jsonl)
     return v < 0 ? 0 : (v > 8 ? 8 : v);
+}
+
+ProofRoute proof_route(uint64_t n, int fk20_capacity, bool eligible) {
+    if (eligible && n <= (uint64_t)direct_proofs_max()) return {true, N_CELLS * (int)n};
+    return {false, fk20_capacity};
+}
+
+const char* item_status_text(uint8_t code, bool cells, bool z) {
+    if (code == ITEM_NON_CANONICAL && cells) return "Serialization(ScalarNotCanonical): a cell field element is >= the scalar modulus";
+    if (code == ITEM_NON_CANONICAL) return "Serialization(ScalarNotCanonical): a blob field element is >= the BLS12-381 scalar modulus";
+    if (code == ITEM_BAD_AUX && z) return "Serialization(ScalarNotCanonical): z is >= the BLS12-381 scalar modulus";
+    if (code == ITEM_BAD_AUX) return "Serialization(G1PointInvalid): commitment is not a valid compressed G1 point in the prime-order subgroup";
+    if (code == ITEM_BAD_DEGREE) return "ReedSolomon(PolynomialHasInvalidLength): recovered polynomial has degree >= 4096";
+    return "Recovery: invalid cell indices";
 }
 
 int chunk_capacity() {
@@ -134,8 +148,7 @@ Status Workspace::ensure_recover_buffers() {
     };
     Status s = all();
     if (!s.ok) {   // all six or none: a half-built set must never be seen by the next borrower of this workspace
-        cudaFree(d_rcells); cudaFreeHost(h_rcells); cudaFree(d_slotmap); cudaFreeHost(h_slotmap); cudaFree(d_ze); cudaFree(d_czinv);
-        d_rcells = nullptr; h_rcells = nullptr; d_slotmap = nullptr; h_slotmap = nullptr; d_ze = nullptr; d_czinv = nullptr;
+        free_recover_buffers();
         cudaGetLastError();
         return s;
     }
@@ -143,8 +156,17 @@ Status Workspace::ensure_recover_buffers() {
     return Status::Ok();
 }
 
-void Workspace::release() {
+void Workspace::free_recover_buffers() {
     cudaFree(d_rcells); cudaFreeHost(h_rcells); cudaFree(d_slotmap); cudaFreeHost(h_slotmap); cudaFree(d_ze); cudaFree(d_czinv);
+    d_rcells = nullptr; h_rcells = nullptr; d_slotmap = nullptr; h_slotmap = nullptr; d_ze = nullptr; d_czinv = nullptr;
+}
+
+void Workspace::synchronize() const {
+    for (cudaStream_t s : {stream, copy_stream, in_stream, aux_stream}) cudaStreamSynchronize(s);
+}
+
+void Workspace::release() {
+    free_recover_buffers();
     cudaFree(d_c48); cudaFree(d_z32); cudaFree(d_out48); cudaFree(d_z); cudaFree(d_aff); cudaFree(d_status2);
     cudaFree(d_blobs); cudaFree(d_coeffs); cudaFree(d_cells); cudaFree(d_scalars); cudaFree(d_pts); cudaFree(d_queue); cudaFree(d_ntt_scratch); cudaFree(d_msm_scratch); cudaFree(d_proofs); cudaFree(d_status);
     cudaFreeHost(h_blobs); cudaFreeHost(h_cells); cudaFreeHost(h_proofs); cudaFreeHost(h_status);
@@ -190,7 +212,6 @@ static Status dev_alloc(std::vector<void*>& allocs, T** p, size_t count) {
     *p = reinterpret_cast<T*>(q);
     return Status::Ok();
 }
-#define EKZG_TRY(expr) do { ::ekzg::Status s_ = (expr); if (!s_.ok) return s_; } while (0)
 
 // device memory the table sizing leaves free for workspaces and other tenants (default 16 GiB)
 static size_t hbm_reserve_bytes() {
@@ -416,7 +437,8 @@ size_t Context::trim_pool(size_t keep) const {
     return victims.size();
 }
 
-void Context::give_back(Workspace* ws) const {
+void Context::give_back(Workspace* ws, const Status& s) const {
+    if (!s.ok) ws->synchronize();
     {
         std::lock_guard<std::mutex> g(pool_mu_);
         pool_.push_back(ws);
@@ -468,18 +490,27 @@ Status Context::proofs_direct_device(Workspace& ws, int n, uint8_t* d_proofs, cu
     return Status::Ok();
 }
 
-Status Context::fk20_from_coeffs_device(Workspace& ws, int n, uint8_t* /*d_cells*/, uint8_t* d_proofs, cudaStream_t stream,
-                                        std::vector<cudaEvent_t>* ev) const {
-    if (!ev && n <= direct_proofs_max() && N_CELLS * n <= ws.capacity) return proofs_direct_device(ws, n, d_proofs, stream);
-    EKZG_CUDA(launch_toeplitz_scalars(ws.d_coeffs, ws.d_scalars, T_, n, stream));
+Status Context::fk20_msm(Workspace& ws, int n, int o, int c, cudaStream_t stream, std::vector<cudaEvent_t>* ev) const {
+    EKZG_CUDA(launch_toeplitz_scalars(ws.d_coeffs, ws.d_scalars, T_, n, stream, o, c));
     if (ev) cudaEventRecord((*ev)[2], stream);
-    EKZG_CUDA(launch_fixed_msm(ws.d_scalars, ws.d_pts, T_.fk20, FK20_MSMS, n, stream, 0, -1, ws.d_msm_scratch));
+    EKZG_CUDA(launch_fixed_msm(ws.d_scalars, ws.d_pts, T_.fk20, FK20_MSMS, n, stream, o, c, ws.d_msm_scratch));
     if (ev) cudaEventRecord((*ev)[3], stream);
+    return Status::Ok();
+}
+
+Status Context::fk20_ntt_compress(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream, std::vector<cudaEvent_t>* ev) const {
     EKZG_CUDA(launch_fk20_g1_ntts(ws.d_pts, n, ws.d_queue, ws.d_ntt_scratch, stream));
     if (ev) cudaEventRecord((*ev)[4], stream);
     EKZG_CUDA(launch_g1_compress(ws.d_pts, d_proofs, N_CELLS, n, stream));
     if (ev) cudaEventRecord((*ev)[5], stream);
     return Status::Ok();
+}
+
+Status Context::fk20_from_coeffs_device(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream, std::vector<cudaEvent_t>* ev) const {
+    const ProofRoute route = proof_route(n, n, !ev);
+    if (route.direct && route.capacity <= ws.capacity) return proofs_direct_device(ws, n, d_proofs, stream);
+    EKZG_TRY(fk20_msm(ws, n, 0, -1, stream, ev));
+    return fk20_ntt_compress(ws, n, d_proofs, stream, ev);
 }
 
 Status Context::fk20_device(Workspace& ws, int n, const uint8_t* d_blobs, uint8_t* d_cells, uint8_t* d_proofs, uint32_t* d_status,
@@ -494,7 +525,7 @@ Status Context::fk20_device(Workspace& ws, int n, const uint8_t* d_blobs, uint8_
     }
     EKZG_CUDA(launch_blob_to_coeffs_cells(d_blobs, ws.d_coeffs, d_cells, d_status, T_, n, d_cells != nullptr, stream));
     if (profiling_ && d_proofs) cudaEventRecord(prof_events_.back()[1], stream);
-    if (d_proofs) EKZG_TRY(fk20_from_coeffs_device(ws, n, d_cells, d_proofs, stream, profiling_ ? &prof_events_.back() : nullptr));
+    if (d_proofs) EKZG_TRY(fk20_from_coeffs_device(ws, n, d_proofs, stream, profiling_ ? &prof_events_.back() : nullptr));
     return Status::Ok();
 }
 
@@ -509,19 +540,20 @@ static bool host_range_is_pinned(const void* p) {
     return a.type == cudaMemoryTypeHost;
 }
 
-// blobs of one chunk -> ws.d_blobs on ws.stream.  Pinned caller memory is DMA'd as it is; pageable memory is copied
-// into the pinned staging buffer in slices, each slice's H2D running while the host copies the next one.
-static Status upload_blobs(Workspace& ws, const uint8_t* src, int cnt, bool src_pinned) {
+// blobs [o, o + cnt) of the chunk at `chunk` -> the same slots of ws.d_blobs, on `st`.  Pinned caller memory is DMA'd as it
+// is; pageable memory is copied into the same slots of the pinned staging buffer in slices, each slice's H2D running while
+// the host copies the next one.
+static Status upload_blobs(Workspace& ws, const uint8_t* chunk, int o, int cnt, bool src_pinned, cudaStream_t st) {
+    const size_t off = (size_t)o * BYTES_PER_BLOB;
     if (src_pinned) {
-        EKZG_CUDA(cudaMemcpyAsync(ws.d_blobs, src, (size_t)cnt * BYTES_PER_BLOB, cudaMemcpyHostToDevice, ws.stream));
+        EKZG_CUDA(cudaMemcpyAsync(ws.d_blobs + off, chunk + off, (size_t)cnt * BYTES_PER_BLOB, cudaMemcpyHostToDevice, st));
         return Status::Ok();
     }
     const int slice = 64;
-    for (int o = 0; o < cnt; o += slice) {
-        const int c = std::min(slice, cnt - o);
-        memcpy(ws.h_blobs + (size_t)o * BYTES_PER_BLOB, src + (size_t)o * BYTES_PER_BLOB, (size_t)c * BYTES_PER_BLOB);
-        EKZG_CUDA(cudaMemcpyAsync(ws.d_blobs + (size_t)o * BYTES_PER_BLOB, ws.h_blobs + (size_t)o * BYTES_PER_BLOB, (size_t)c * BYTES_PER_BLOB,
-                                  cudaMemcpyHostToDevice, ws.stream));
+    for (int i = 0; i < cnt; i += slice) {
+        const size_t at = off + (size_t)i * BYTES_PER_BLOB, bytes = (size_t)std::min(slice, cnt - i) * BYTES_PER_BLOB;
+        memcpy(ws.h_blobs + at, chunk + at, bytes);
+        EKZG_CUDA(cudaMemcpyAsync(ws.d_blobs + at, ws.h_blobs + at, bytes, cudaMemcpyHostToDevice, st));
     }
     return Status::Ok();
 }
@@ -539,16 +571,16 @@ Status Context::compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* bl
     EKZG_TRY(bind_device());
     const int cap = (int)std::min<uint64_t>(n, (uint64_t)chunk_capacity());
     const uint64_t nchunks = (n + cap - 1) / cap;
-    const bool direct = want_proofs && n <= (uint64_t)direct_proofs_max();   // latency path: see proofs_direct_device
-    Workspace* W[2] = {acquire(direct ? N_CELLS * (int)n : cap, true), nchunks > 1 ? acquire(cap, true) : nullptr};
+    const ProofRoute route = proof_route(n, cap, want_proofs);   // direct: the latency path, see proofs_direct_device
+    Workspace* W[2] = {acquire(route.capacity, true), nchunks > 1 ? acquire(cap, true) : nullptr};
     if (!W[0] || (nchunks > 1 && !W[1])) {
-        for (Workspace* w : W) if (w) give_back(w);
-        return Status::Error("device/pinned memory allocation failed");
+        const Status s = Status::Error("device/pinned memory allocation failed");
+        for (Workspace* w : W) if (w) give_back(w, s);
+        return s;
     }
     const bool in_pinned = host_range_is_pinned(blobs);
     const bool cells_pinned = cells && host_range_is_pinned(cells);
     const bool proofs_pinned = want_proofs && host_range_is_pinned(proofs);
-    constexpr size_t CELLS_PER_BLOB = (size_t)N_EXT * 32, PROOFS_PER_BLOB = (size_t)N_CELLS * BYTES_PER_G1;
     bool any_bad = false;
     Status result = Status::Ok();
     TraceClock tr("compute_cells_and_kzg_proofs_batch");
@@ -582,7 +614,7 @@ Status Context::compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* bl
         if (want_proofs && !proofs_pinned) memcpy(proofs + first * PROOFS_PER_BLOB, ws.h_proofs, (size_t)cnt * PROOFS_PER_BLOB);
         for (int i = 0; i < cnt; i++) {
             if (ws.h_status[i]) any_bad = true;
-            if (blob_status) blob_status[first + i] = ws.h_status[i] ? 1 : 0;
+            if (blob_status) blob_status[first + i] = ws.h_status[i] ? ITEM_NON_CANONICAL : ITEM_OK;
         }
         pending_cnt[slot] = 0;
         return Status::Ok();
@@ -611,17 +643,7 @@ Status Context::compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* bl
         EKZG_CUDA(cudaMemsetAsync(ws.d_status, 0, sizeof(uint32_t) * cnt, ws.stream));
         for (int s = 0; s < np; s++) {
             const int o = off[s], c = len[s];
-            if (in_pinned) {
-                EKZG_CUDA(cudaMemcpyAsync(ws.d_blobs + (size_t)o * BYTES_PER_BLOB, blobs + (first + o) * BYTES_PER_BLOB, (size_t)c * BYTES_PER_BLOB,
-                                          cudaMemcpyHostToDevice, ws.in_stream));
-            } else {   // pageable caller memory: through the pinned staging buffer in slices, each slice's DMA under the next host copy
-                for (int i = 0; i < c; i += 64) {
-                    const int cc = std::min(64, c - i);
-                    uint8_t* stage = ws.h_blobs + (size_t)(o + i) * BYTES_PER_BLOB;
-                    memcpy(stage, blobs + (first + o + i) * BYTES_PER_BLOB, (size_t)cc * BYTES_PER_BLOB);
-                    EKZG_CUDA(cudaMemcpyAsync(ws.d_blobs + (size_t)(o + i) * BYTES_PER_BLOB, stage, (size_t)cc * BYTES_PER_BLOB, cudaMemcpyHostToDevice, ws.in_stream));
-                }
-            }
+            EKZG_TRY(upload_blobs(ws, blobs + first * BYTES_PER_BLOB, o, c, in_pinned, ws.in_stream));
             stamp("H2D done, piece", s, ws.in_stream);
             EKZG_CUDA(cudaEventRecord(ws.piece_in[s], ws.in_stream));
             EKZG_CUDA(cudaStreamWaitEvent(ws.stream, ws.piece_in[s], 0));
@@ -635,20 +657,17 @@ Status Context::compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* bl
                 EKZG_CUDA(cudaMemcpyAsync(dst, ws.d_cells + (size_t)o * CELLS_PER_BLOB, (size_t)c * CELLS_PER_BLOB, cudaMemcpyDeviceToHost, ws.copy_stream));
                 EKZG_CUDA(cudaEventRecord(ws.sub_out[s], ws.copy_stream));
             }
-            if (want_proofs && !direct) {
-                EKZG_CUDA(launch_toeplitz_scalars(ws.d_coeffs, ws.d_scalars, T_, cnt, ws.stream, o, c));
-                EKZG_CUDA(launch_fixed_msm(ws.d_scalars, ws.d_pts, T_.fk20, FK20_MSMS, cnt, ws.stream, o, c, ws.d_msm_scratch));
+            if (want_proofs && !route.direct) {
+                EKZG_TRY(fk20_msm(ws, cnt, o, c, ws.stream, nullptr));
                 stamp("K4 done, piece", s, ws.stream);
             }
         }
         if (want_proofs) {
-            if (direct) {
+            if (route.direct) {
                 EKZG_TRY(proofs_direct_device(ws, cnt, ws.d_proofs, ws.stream));
                 stamp("direct proofs done", -1, ws.stream);
             } else {
-                EKZG_CUDA(launch_fk20_g1_ntts(ws.d_pts, cnt, ws.d_queue, ws.d_ntt_scratch, ws.stream));
-                stamp("K5 done", -1, ws.stream);
-                EKZG_CUDA(launch_g1_compress(ws.d_pts, ws.d_proofs, N_CELLS, cnt, ws.stream));
+                EKZG_TRY(fk20_ntt_compress(ws, cnt, ws.d_proofs, ws.stream, nullptr));
             }
             EKZG_CUDA(cudaMemcpyAsync(proofs_pinned ? proofs + first * PROOFS_PER_BLOB : ws.h_proofs, ws.d_proofs, (size_t)cnt * PROOFS_PER_BLOB,
                                       cudaMemcpyDeviceToHost, ws.stream));
@@ -672,8 +691,7 @@ Status Context::compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* bl
     for (int slot = 0; slot < 2; slot++) {
         if (!W[slot]) continue;
         if (result.ok) result = drain(slot);
-        if (!result.ok) { cudaStreamSynchronize(W[slot]->in_stream); cudaStreamSynchronize(W[slot]->stream); cudaStreamSynchronize(W[slot]->copy_stream); }
-        give_back(W[slot]);
+        give_back(W[slot], result);
     }
     if (tr.on && !tl.empty()) {
         cudaDeviceSynchronize();
@@ -686,7 +704,7 @@ Status Context::compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* bl
         for (auto& pe : tl) cudaEventDestroy(pe.second);
     }
     if (!result.ok) return result;
-    if (any_bad) return Status::Error("Serialization(ScalarNotCanonical): a blob field element is >= the BLS12-381 scalar modulus");
+    if (any_bad) return Status::Error(item_status_text(ITEM_NON_CANONICAL, false, false));
     return Status::Ok();
 }
 
@@ -724,16 +742,13 @@ void Context::CoalesceStaging::release() {
     in = cells = proofs = nullptr;
 }
 
-static Status item_error(int which_recover, uint8_t code) {
-    if (!which_recover) return Status::Error("Serialization(ScalarNotCanonical): a blob field element is >= the BLS12-381 scalar modulus");
-    if (code == 1) return Status::Error("Serialization(ScalarNotCanonical): a cell field element is >= the scalar modulus");
-    if (code == 4) return Status::Error("ReedSolomon(PolynomialHasInvalidLength): recovered polynomial has degree >= 4096");
-    return Status::Error("Recovery: invalid cell indices");
+// 128 cells or proofs of one blob, contiguous at `src`, out through the 128 separate pointers the C ABI hands over
+static void scatter(const uint8_t* src, size_t item_bytes, uint8_t* const* dst) {
+    for (int i = 0; i < N_CELLS; i++) memcpy(dst[i], src + (size_t)i * item_bytes, item_bytes);
 }
 
 Status Context::coalesce(int which, CoalesceReq& me) const {
     CoalesceQueue& Q = co_[which];
-    constexpr size_t CELLS_PER_BLOB = (size_t)N_EXT * 32, PROOFS_PER_BLOB = (size_t)N_CELLS * BYTES_PER_G1;
     const bool recover = which == CQ_RECOVER, want_proofs = which != CQ_CELLS;
     const int cap = coalesce_capacity();
     static const int linger_us = [] { const char* e = getenv("EKZG_COALESCE_LINGER_US"); return e ? atoi(e) : 300; }();
@@ -782,8 +797,6 @@ Status Context::coalesce(int which, CoalesceReq& me) const {
     }
     const int slot = Bt->n++;
     Bt->left++;
-    size_t cell_off = 0;
-    if (recover) { cell_off = Bt->cells_total; Bt->cells_total += me.count; }
     CoalesceStaging& st = *Bt->st;
     lk.unlock();
     // ---- copy my input into my slot (all members do this at the same time) ----
@@ -796,7 +809,6 @@ Status Context::coalesce(int which, CoalesceReq& me) const {
     } else {
         memcpy(st.in + (size_t)slot * st.in_stride, me.in, BYTES_PER_BLOB);
     }
-    (void)cell_off;
     lk.lock();
     Bt->copied++;
     Q.cv_leader.notify_all();
@@ -831,7 +843,7 @@ Status Context::coalesce(int which, CoalesceReq& me) const {
             // other batches are on the device already (or the next one is forming behind this one): this batch cannot have the
             // device to itself, so ask for the G1-NTT kernel with the least work (kzg_kernels.h) instead of the latency-mode ones
             set_k5_throughput_hint(crowded);
-            if (recover) s = recover_cells_and_kzg_proofs_strided(n, st.counts.data(), st.indices.data(), st.in, st.cells, st.proofs, st.status.data());
+            if (recover) s = recover_impl(n, st.counts.data(), st.indices.data(), st.in, st.cells, st.proofs, st.status.data(), true);
             else s = compute_cells_and_kzg_proofs_batch(n, st.in, st.cells, want_proofs ? st.proofs : nullptr, st.status.data(), want_proofs);
         } catch (const std::exception& ex) {             // fail the batch, never the queue
             s = Status::Error(std::string("batch failed: ") + ex.what());
@@ -859,14 +871,14 @@ Status Context::coalesce(int which, CoalesceReq& me) const {
     if (!Bt->result.ok && !any_flag) {
         mine = Bt->result;                                // the batch as a whole failed (CUDA error, allocation)
     } else if (st.status[slot]) {
-        mine = item_error(recover, st.status[slot]);      // this item is the invalid one; the others are served
+        mine = Status::Error(item_status_text(st.status[slot], recover, false));   // this item is the invalid one; the others are served
     } else {
         const uint8_t* c = st.cells + (size_t)slot * CELLS_PER_BLOB;
-        if (me.cells_scattered) for (int i = 0; i < N_CELLS; i++) memcpy(me.cells_scattered[i], c + (size_t)i * BYTES_PER_CELL, BYTES_PER_CELL);
+        if (me.cells_scattered) scatter(c, BYTES_PER_CELL, me.cells_scattered);
         else memcpy(me.cells, c, CELLS_PER_BLOB);
         if (want_proofs) {
             const uint8_t* p = st.proofs + (size_t)slot * PROOFS_PER_BLOB;
-            if (me.proofs_scattered) for (int i = 0; i < N_CELLS; i++) memcpy(me.proofs_scattered[i], p + (size_t)i * BYTES_PER_G1, BYTES_PER_G1);
+            if (me.proofs_scattered) scatter(p, BYTES_PER_G1, me.proofs_scattered);
             else memcpy(me.proofs, p, PROOFS_PER_BLOB);
         }
     }
@@ -884,19 +896,27 @@ static bool coalescing_off() {
     return off;
 }
 
+// One item as a batch of one, past the coalescer: run(cells, proofs) is the batch call, and outputs bound for 128 separate
+// pointers go through temporary contiguous buffers.
+template <class Run>
+static Status run_uncoalesced(uint8_t* cells, uint8_t* proofs, uint8_t* const* cells_scattered, uint8_t* const* proofs_scattered, Run run) {
+    std::vector<uint8_t> tc(cells_scattered ? CELLS_PER_BLOB : 0), tp(proofs_scattered ? PROOFS_PER_BLOB : 0);
+    if (cells_scattered) cells = tc.data();
+    if (proofs_scattered) proofs = tp.data();
+    Status s = run(cells, proofs);
+    if (!s.ok) return s;
+    if (cells_scattered) scatter(cells, BYTES_PER_CELL, cells_scattered);
+    if (proofs_scattered) scatter(proofs, BYTES_PER_G1, proofs_scattered);
+    return s;
+}
+
 Status Context::compute_cells_and_kzg_proofs_one(const uint8_t* blob, uint8_t* cells, uint8_t* proofs, uint8_t* const* cells_scattered,
                                                  uint8_t* const* proofs_scattered, bool want_proofs) const {
-    if (coalescing_off()) {
-        constexpr size_t CELLS_PER_BLOB = (size_t)N_EXT * 32, PROOFS_PER_BLOB = (size_t)N_CELLS * BYTES_PER_G1;
-        std::vector<uint8_t> tc, tp;
-        if (cells_scattered) { tc.resize(CELLS_PER_BLOB); cells = tc.data(); }
-        if (want_proofs && proofs_scattered) { tp.resize(PROOFS_PER_BLOB); proofs = tp.data(); }
-        Status s = compute_cells_and_kzg_proofs_batch(1, blob, cells, want_proofs ? proofs : nullptr, nullptr, want_proofs);
-        if (!s.ok) return s;
-        if (cells_scattered) for (int i = 0; i < N_CELLS; i++) memcpy(cells_scattered[i], cells + (size_t)i * BYTES_PER_CELL, BYTES_PER_CELL);
-        if (want_proofs && proofs_scattered) for (int i = 0; i < N_CELLS; i++) memcpy(proofs_scattered[i], proofs + (size_t)i * BYTES_PER_G1, BYTES_PER_G1);
-        return s;
-    }
+    if (!want_proofs) { proofs = nullptr; proofs_scattered = nullptr; }
+    if (coalescing_off())
+        return run_uncoalesced(cells, proofs, cells_scattered, proofs_scattered, [&](uint8_t* c, uint8_t* p) {
+            return compute_cells_and_kzg_proofs_batch(1, blob, c, p, nullptr, want_proofs);
+        });
     CoalesceReq me;
     me.in = blob; me.cells = cells; me.proofs = proofs; me.cells_scattered = cells_scattered; me.proofs_scattered = proofs_scattered;
     return coalesce(want_proofs ? CQ_CELLS_PROOFS : CQ_CELLS, me);
@@ -908,17 +928,10 @@ Status Context::recover_cells_and_kzg_proofs_one(uint64_t count, const uint64_t*
     // malformed request never joins a shared batch
     bool bad = count < (uint64_t)N_CELLS / 2 || count > (uint64_t)N_CELLS;
     for (uint64_t k = 0; k < count && !bad; k++) bad = indices[k] >= (uint64_t)N_CELLS || (k && !(indices[k - 1] < indices[k]));
-    if (bad || coalescing_off()) {
-        constexpr size_t CELLS_PER_BLOB = (size_t)N_EXT * 32, PROOFS_PER_BLOB = (size_t)N_CELLS * BYTES_PER_G1;
-        std::vector<uint8_t> tc, tp;
-        if (cells_scattered) { tc.resize(CELLS_PER_BLOB); out_cells = tc.data(); }
-        if (proofs_scattered) { tp.resize(PROOFS_PER_BLOB); out_proofs = tp.data(); }
-        Status s = recover_cells_and_kzg_proofs_batch(1, &count, indices, cells, out_cells, out_proofs, nullptr);
-        if (!s.ok) return s;
-        if (cells_scattered) for (int i = 0; i < N_CELLS; i++) memcpy(cells_scattered[i], out_cells + (size_t)i * BYTES_PER_CELL, BYTES_PER_CELL);
-        if (proofs_scattered) for (int i = 0; i < N_CELLS; i++) memcpy(proofs_scattered[i], out_proofs + (size_t)i * BYTES_PER_G1, BYTES_PER_G1);
-        return s;
-    }
+    if (bad || coalescing_off())
+        return run_uncoalesced(out_cells, out_proofs, cells_scattered, proofs_scattered, [&](uint8_t* c, uint8_t* p) {
+            return recover_cells_and_kzg_proofs_batch(1, &count, indices, cells, c, p, nullptr);
+        });
     CoalesceReq me;
     me.in = cells; me.indices = indices; me.count = count; me.cells = out_cells; me.proofs = out_proofs;
     me.cells_scattered = cells_scattered; me.proofs_scattered = proofs_scattered;
@@ -936,11 +949,6 @@ static int rev7(int x) {
 Status Context::recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
                                                    uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const {
     return recover_impl(n, counts, indices, cells, out_cells, out_proofs, item_status, false);
-}
-// the same with item i's indices at indices + 128 i and its cells at cells + 128 i * 2048 (the coalescer's staging slots)
-Status Context::recover_cells_and_kzg_proofs_strided(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
-                                                     uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const {
-    return recover_impl(n, counts, indices, cells, out_cells, out_proofs, item_status, true);
 }
 
 Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells, uint8_t* out_cells,
@@ -963,20 +971,18 @@ Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t*
         if (!err && c < (uint64_t)N_CELLS / 2) err = "Recovery(NotEnoughCellsToReconstruct)";
         if (!err && c > (uint64_t)N_CELLS) err = "Recovery(TooManyCellsReceived)";
         if (err) {
-            code[i] = 3;
+            code[i] = ITEM_BAD_INDICES;
             if (first_err.empty()) first_err = err;
         }
     }
     const int cap = (int)std::min<uint64_t>(n, (uint64_t)chunk_capacity());
-    // (one or two blobs: room for the direct proof path, 128 virtual blobs per blob)
-    Workspace* wsp = acquire(n <= (uint64_t)direct_proofs_max() ? N_CELLS * (int)n : cap, true);
+    Workspace* wsp = acquire(proof_route(n, cap, true).capacity, true);
     if (!wsp) return Status::Error("device/pinned memory allocation failed");
     Workspace& ws = *wsp;
     Status result = ws.ensure_recover_buffers();
     if (!result.ok) { discard(wsp); return result; }
     cudaStream_t st = ws.stream;
     const bool in_pinned = host_range_is_pinned(cells), cells_pinned = host_range_is_pinned(out_cells), proofs_pinned = host_range_is_pinned(out_proofs);
-    constexpr size_t CELLS_PER_BLOB = (size_t)N_EXT * 32, PROOFS_PER_BLOB = (size_t)N_CELLS * BYTES_PER_G1;
     TraceClock tr("recover_cells_and_kzg_proofs_batch");
     auto body = [&](uint64_t first, int cnt) -> Status {
         // slot maps (which input cell sits at which bit-reversed position) and the cells themselves: blob i's cells go
@@ -1014,7 +1020,7 @@ Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t*
         EKZG_CUDA(cudaMemcpyAsync(cells_pinned ? out_cells + first * CELLS_PER_BLOB : ws.h_cells, ws.d_cells, (size_t)cnt * CELLS_PER_BLOB,
                                   cudaMemcpyDeviceToHost, ws.copy_stream));
         EKZG_CUDA(cudaEventRecord(ws.sub_out[0], ws.copy_stream));
-        EKZG_TRY(fk20_from_coeffs_device(ws, cnt, ws.d_cells, ws.d_proofs, st));
+        EKZG_TRY(fk20_from_coeffs_device(ws, cnt, ws.d_proofs, st));
         EKZG_CUDA(cudaMemcpyAsync(proofs_pinned ? out_proofs + first * PROOFS_PER_BLOB : ws.h_proofs, ws.d_proofs, (size_t)cnt * PROOFS_PER_BLOB,
                                   cudaMemcpyDeviceToHost, st));
         EKZG_CUDA(cudaMemcpyAsync(ws.h_status, ws.d_status, sizeof(uint32_t) * cnt, cudaMemcpyDeviceToHost, st));
@@ -1026,17 +1032,14 @@ Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t*
         for (int i = 0; i < cnt; i++) {
             const uint64_t g = first + i;
             if (!code[g] && ws.h_status[i]) {
-                code[g] = (ws.h_status[i] & 1) ? 1 : 4;
-                if (first_err.empty())
-                    first_err = (ws.h_status[i] & 1) ? "Serialization(ScalarNotCanonical): a cell field element is >= the scalar modulus"
-                                                     : "ReedSolomon(PolynomialHasInvalidLength): recovered polynomial has degree >= 4096";
+                code[g] = (ws.h_status[i] & 1) ? ITEM_NON_CANONICAL : ITEM_BAD_DEGREE;
+                if (first_err.empty()) first_err = item_status_text(code[g], true, false);
             }
         }
         return Status::Ok();
     };
     for (uint64_t first = 0; first < n && result.ok; first += cap) result = body(first, (int)std::min<uint64_t>(cap, n - first));
-    if (!result.ok) { cudaStreamSynchronize(st); cudaStreamSynchronize(ws.copy_stream); }
-    give_back(wsp);
+    give_back(wsp, result);
     if (item_status) memcpy(item_status, code.data(), n);
     if (!result.ok) return result;
     if (!first_err.empty()) return Status::Error(first_err);
@@ -1069,7 +1072,7 @@ Status Context::run_4844(Mode4844 mode, uint64_t n, const uint8_t* blobs, const 
             EKZG_CUDA(launch_g1_validate(ws.d_c48, ws.d_aff, ws.d_status2, cnt, true, ws.copy_stream));
             EKZG_CUDA(cudaEventRecord(ws.sub_out[0], ws.copy_stream));
         }
-        EKZG_TRY(upload_blobs(ws, blobs + first * BYTES_PER_BLOB, cnt, in_pinned));
+        EKZG_TRY(upload_blobs(ws, blobs + first * BYTES_PER_BLOB, 0, cnt, in_pinned, st));
         tr.mark("stage + enqueue H2D of the blobs");
         EKZG_CUDA(cudaMemsetAsync(ws.d_status, 0, sizeof(uint32_t) * cnt, st));
         if (mode != Mode4844::BlobProof) EKZG_CUDA(cudaMemsetAsync(ws.d_status2, 0, sizeof(uint32_t) * cnt, st));
@@ -1103,21 +1106,18 @@ Status Context::run_4844(Mode4844 mode, uint64_t n, const uint8_t* blobs, const 
         EKZG_CUDA(cudaStreamSynchronize(st));
         tr.mark("H2D + kernels + D2H");
         for (int i = 0; i < cnt; i++) {
-            uint8_t code = hs[i] ? 1 : (hs2[i] ? 2 : 0);
-            if (code == 1) bad_blob = true;
-            if (code == 2) bad_aux = true;
+            const uint8_t code = hs[i] ? ITEM_NON_CANONICAL : (hs2[i] ? ITEM_BAD_AUX : ITEM_OK);
+            if (code == ITEM_NON_CANONICAL) bad_blob = true;
+            if (code == ITEM_BAD_AUX) bad_aux = true;
             if (item_status) item_status[first + i] = code;
         }
         return Status::Ok();
     };
     for (uint64_t first = 0; first < n && result.ok; first += cap) result = body(first, (int)std::min<uint64_t>(cap, n - first));
-    if (!result.ok) { cudaStreamSynchronize(st); cudaStreamSynchronize(ws.copy_stream); }
-    give_back(wsp);
+    give_back(wsp, result);
     if (!result.ok) return result;
-    if (bad_blob) return Status::Error("Serialization(ScalarNotCanonical): a blob field element is >= the BLS12-381 scalar modulus");
-    if (bad_aux)
-        return Status::Error(mode == Mode4844::BlobProof ? "Serialization(G1PointInvalid): commitment is not a valid compressed G1 point in the prime-order subgroup"
-                                                         : "Serialization(ScalarNotCanonical): z is >= the BLS12-381 scalar modulus");
+    if (bad_blob) return Status::Error(item_status_text(ITEM_NON_CANONICAL, false, false));
+    if (bad_aux) return Status::Error(item_status_text(ITEM_BAD_AUX, false, mode == Mode4844::PointProof));
     return Status::Ok();
 }
 

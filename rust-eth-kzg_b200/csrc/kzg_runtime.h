@@ -27,6 +27,19 @@ struct Status {
         cudaError_t e_ = (expr);                                                                                \
         if (e_ != cudaSuccess) return ::ekzg::Status::Error(std::string("CUDA error: ") + cudaGetErrorString(e_) + " at " #expr); \
     } while (0)
+#define EKZG_TRY(expr) do { ::ekzg::Status s_ = (expr); if (!s_.ok) return s_; } while (0)
+
+// Per-item status codes of the batch calls (item_status / blob_status of the C ABI: the values are fixed).
+enum ItemStatus : uint8_t {
+    ITEM_OK = 0,
+    ITEM_NON_CANONICAL = 1,   // a blob or cell field element is >= the scalar modulus
+    ITEM_BAD_AUX = 2,         // compute_blob_kzg_proof: invalid commitment; compute_kzg_proof: non-canonical z
+    ITEM_BAD_INDICES = 3,     // recovery: cell indices out of range, not ascending, too few or too many
+    ITEM_BAD_DEGREE = 4,      // recovery: the recovered polynomial has degree >= 4096
+};
+// The error text of an item with status `code`: `cells` -- its inputs were cells (recovery), not a blob; `z` -- its second
+// input was an evaluation point, not a commitment.
+const char* item_status_text(uint8_t code, bool cells, bool z);
 
 // A caller-supplied trusted setup with its points still in compressed form: what TrustedSetup::from_json /
 // from_json_unchecked (crates/trusted_setup/src/lib.rs:112-127) hand to DASContext::new (crates/eip7594/src/lib.rs).
@@ -78,14 +91,24 @@ struct Workspace {
     Fr* d_czinv = nullptr;
     bool recover_ready = false;    // all six recovery buffers exist
     Status ensure_recover_buffers();
+    void free_recover_buffers();
     // pinned host staging (the ABI hands us scattered caller buffers)
     uint8_t* h_blobs = nullptr;
     uint8_t* h_cells = nullptr;
     uint8_t* h_proofs = nullptr;
     uint32_t* h_status = nullptr;
     Status alloc(int cap, bool with_io, size_t msm_scratch_bytes);
+    void synchronize() const;   // waits for the work queued on all four streams
     void release();
 };
+
+// Proof route of an n-blob call.  Up to EKZG_DIRECT_MAX blobs (default 1, 0 = off) take the DIRECT route (128 SRS MSMs per
+// blob instead of FK20) when `eligible` (the call computes proofs and is not timed per FK20 stage).
+struct ProofRoute {
+    bool direct;
+    int capacity;   // workspace capacity the call needs: 128 "virtual blobs" per blob on the direct route, else `fk20_capacity`
+};
+ProofRoute proof_route(uint64_t n, int fk20_capacity, bool eligible);
 
 class Context {
 public:
@@ -99,14 +122,9 @@ public:
     uint64_t table_bytes() const { return table_bytes_; }
     const host::G2Keys* g2_keys() const { return g2keys_; }
 
-    // Everything on device, asynchronous on `stream`; scratch comes from `ws` (capacity >= n).
+    // Everything on device, asynchronous on `stream`; scratch comes from `ws` (capacity: proof_route(n, n, d_proofs).capacity).
     Status fk20_device(Workspace& ws, int n, const uint8_t* d_blobs, uint8_t* d_cells, uint8_t* d_proofs, uint32_t* d_status,
                        cudaStream_t stream) const;
-    // same, starting from coefficients already in ws.d_coeffs (recovery path)
-    // proofs of n <= direct_proofs_max() blobs from ws.d_coeffs by the direct route (needs ws.capacity >= 128 n)
-    Status proofs_direct_device(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream) const;
-    Status fk20_from_coeffs_device(Workspace& ws, int n, uint8_t* d_cells, uint8_t* d_proofs, cudaStream_t stream,
-                                   std::vector<cudaEvent_t>* stage_events = nullptr) const;
 
     // Host buffers, contiguous; chunks the batch through two workspaces.
     Status compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* blobs, uint8_t* cells, uint8_t* proofs,
@@ -126,7 +144,7 @@ public:
                                             uint8_t* out_proofs, uint8_t* const* cells_scattered, uint8_t* const* proofs_scattered) const;
 
     // EIP-4844 prover side (crates/eip4844/src/prover.rs:17-88), batched.  Host buffers, contiguous.
-    // item_status[i]: 0 ok, 1 invalid blob, 2 invalid commitment / z.
+    // item_status[i]: ItemStatus 0, 1 or 2.
     Status blob_to_kzg_commitment_batch(uint64_t n, const uint8_t* blobs, uint8_t* out48, uint8_t* item_status) const;
     Status compute_blob_kzg_proof_batch(uint64_t n, const uint8_t* blobs, const uint8_t* commitments48, uint8_t* out48,
                                         uint8_t* item_status) const;
@@ -134,8 +152,8 @@ public:
                                    uint8_t* item_status) const;
 
     // Erasure recovery (crates/eip7594/src/prover.rs:156-171, recovery.rs:22-146), batched: blob i provides counts[i]
-    // cells; indices and cells of all blobs are concatenated.  item_status: 0 ok, 3 invalid indices, 1 non-canonical
-    // cell scalar, 4 recovered polynomial of too high degree.  out_* contiguous per blob (128*2048 B, 128*48 B).
+    // cells; indices and cells of all blobs are concatenated.  item_status: ItemStatus 0, 1, 3 or 4.
+    // out_* contiguous per blob (128*2048 B, 128*48 B).
     Status recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
                                               uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const;
 
@@ -149,7 +167,9 @@ public:
 
     // workspace pool (calls are re-entrant: concurrent callers each borrow their own workspaces)
     Workspace* acquire(int min_capacity, bool with_io) const;
-    void give_back(Workspace* ws) const;
+    // `s`: the outcome of the call that borrowed `ws`.  After a failure the work queued before it may still be running: the
+    // workspace's streams are synchronised before it is pooled, so the next borrower finds its buffers idle.
+    void give_back(Workspace* ws, const Status& s) const;
     void discard(Workspace* ws) const;             // destroy instead of pooling (its buffers are incomplete)
     size_t trim_pool(size_t keep) const;           // release idle workspaces beyond `keep`
 
@@ -168,6 +188,14 @@ private:
     Status run_4844(Mode4844 mode, uint64_t n, const uint8_t* blobs, const uint8_t* aux_in, uint8_t* out48, uint8_t* out_y32,
                     uint8_t* item_status) const;
     Context() = default;
+    // proofs of n blobs from ws.d_coeffs, asynchronous on `stream`: by the direct route when proof_route() picks it
+    // (never with stage_events), else FK20 = fk20_msm of all n blobs, then fk20_ntt_compress
+    Status fk20_from_coeffs_device(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream,
+                                   std::vector<cudaEvent_t>* stage_events = nullptr) const;
+    Status proofs_direct_device(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream) const;   // needs ws.capacity >= 128 n
+    // K2 + K4 of blobs [o, o + c) of an n-blob batch (c < 0: to the end), then K5 + K6 of all n; stage events 2..5 as in fk20_device
+    Status fk20_msm(Workspace& ws, int n, int o, int c, cudaStream_t stream, std::vector<cudaEvent_t>* stage_events) const;
+    Status fk20_ntt_compress(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream, std::vector<cudaEvent_t>* stage_events) const;
     // Leader/follower coalescing of concurrent single-item callers into shared batches (see compute_cells_and_kzg_proofs_one).
     struct CoalesceReq {
         // compute: blob -> cells (+ proofs);   recover: count cells at `indices` -> cells + proofs
@@ -196,7 +224,6 @@ private:
         int n = 0;          // members that joined
         int copied = 0;     // members whose input is in the block
         int left = 0;       // members that have not copied their results out yet
-        size_t cells_total = 0;
         bool closed = false, done = false;
         Status result = Status::Ok();
     };
@@ -213,10 +240,9 @@ private:
     enum { CQ_CELLS = 0, CQ_CELLS_PROOFS = 1, CQ_RECOVER = 2 };
     mutable CoalesceQueue co_[3];
     Status coalesce(int which, CoalesceReq& me) const;
+    // strided: item i's indices at indices + 128 i and its cells at cells + 128 i * 2048 (the coalescer's staging slots)
     Status recover_impl(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells, uint8_t* out_cells, uint8_t* out_proofs,
                         uint8_t* item_status, bool strided) const;
-    Status recover_cells_and_kzg_proofs_strided(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
-                                                uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const;
     Status init(bool use_precomp, int device, const SetupBytes* custom);
     host::G2Keys* g2keys_ = nullptr;   // G2 side of a caller-supplied setup (nullptr: the embedded ceremony's constants)
     int device_ = 0;
@@ -233,9 +259,6 @@ private:
 };
 
 int chunk_capacity();
-// up to this many blobs per call take the DIRECT proof path (128 SRS MSMs per blob instead of the FK20 route; EKZG_DIRECT_MAX, 0 = off);
-// a workspace must hold 128 "virtual blobs" per blob for it
-int direct_proofs_max();
 // z = SHA-256("FSBLOBVERIFY_V1_" || u128_be(4096) || blob || commitment) mod r as 32 canonical big-endian bytes
 // (crates/eip4844/src/verifier.rs:155-196) on the HOST: for a handful of blobs the x86 SHA extensions (0.1 ms per blob) beat the
 // device kernel, where one thread walks the 2049 compressions of a blob (~4 ms whatever the count).

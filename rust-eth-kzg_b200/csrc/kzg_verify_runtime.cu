@@ -14,8 +14,6 @@
 
 namespace ekzg {
 
-#define EKZG_TRY(expr) do { ::ekzg::Status s_ = (expr); if (!s_.ok) return s_; } while (0)
-
 namespace {
 
 // stream-ordered scratch that frees itself
@@ -232,9 +230,9 @@ Status Context::verify_cell_kzg_proof_batch(uint64_t n_commitments, const uint8_
             return Status::Ok();
         };
         result = run();
-        if (!result.ok) { cudaStreamSynchronize(wsp->copy_stream); cudaStreamSynchronize(wsp->in_stream); cudaStreamSynchronize(wsp->aux_stream); cudaStreamSynchronize(st); }
+        if (!result.ok) wsp->synchronize();   // S frees in the order of `st` alone: the side streams' work must be over first
     }
-    give_back(wsp);
+    give_back(wsp, result);
     if (!result.ok) return result;
     // deserialisation errors in the reference's order: commitments, proofs, cells (verifier.rs:96-98)
     for (uint32_t v : stc) if (v) return Status::Error("Serialization(G1PointInvalid): commitment");
@@ -363,9 +361,9 @@ Status Context::verify_kzg_proofs(int mode, uint64_t n, const uint8_t* const* bl
             return Status::Ok();
         };
         result = run();
-        if (!result.ok) { cudaStreamSynchronize(ws.copy_stream); cudaStreamSynchronize(st); }
+        if (!result.ok) ws.synchronize();     // (see verify_cell_kzg_proof_batch)
     }
-    give_back(wsp);
+    give_back(wsp, result);
     if (!result.ok) return result;
     for (uint32_t v : stb) if (v) return Status::Error("Serialization(ScalarNotCanonical): blob");
     for (uint32_t v : stc) if (v) return Status::Error("Serialization(G1PointInvalid): commitment");

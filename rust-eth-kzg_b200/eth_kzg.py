@@ -80,6 +80,17 @@ def _check(lib, res):
         raise KzgError(msg)
 
 
+def _batch_status(lib, res, status, n):
+    """the status list of a batch call; raises KzgError when the call failed and no item is flagged (an infrastructure error)"""
+    st = list(status.raw[:n])
+    if res.status != 0:
+        msg = C.string_at(res.error_msg).decode("utf-8", "replace") if res.error_msg else ""
+        lib.eth_kzg_free_error_message(res.error_msg)
+        if not any(st):
+            raise KzgError("batch failed: " + msg)
+    return st
+
+
 def _exact(b, n, what):
     """the reference's API takes fixed-size array references; a wrong length cannot cross its FFI either"""
     if len(b) != n:
@@ -255,12 +266,7 @@ class DASContext:
         proofs = C.create_string_buffer(n * CELLS_PER_EXT_BLOB * 48) if want_proofs else None
         status = C.create_string_buffer(max(n, 1))
         res = self._lib.eth_kzg_b200_compute_cells_and_kzg_proofs_batch(C.c_void_p(self._ctx), C.c_uint64(n), blobs_flat, cells, proofs, status)
-        st = list(status.raw[:n])
-        if res.status != 0:
-            msg = C.string_at(res.error_msg).decode("utf-8", "replace") if res.error_msg else ""
-            self._lib.eth_kzg_free_error_message(res.error_msg)
-            if not any(st):
-                raise KzgError("batch failed: " + msg)
+        st = _batch_status(self._lib, res, status, n)
         return cells.raw, (proofs.raw if want_proofs else None), st
 
     def blob_to_kzg_commitment_batch(self, blobs_flat, n):
@@ -268,11 +274,7 @@ class DASContext:
         out = C.create_string_buffer(max(n, 1) * 48)
         status = C.create_string_buffer(max(n, 1))
         res = self._lib.eth_kzg_b200_blob_to_kzg_commitment_batch(C.c_void_p(self._ctx), C.c_uint64(n), _exact(blobs_flat, n * BYTES_PER_BLOB, "blobs"), out, status)
-        st = list(status.raw[:n])
-        if res.status != 0:
-            self._lib.eth_kzg_free_error_message(res.error_msg)
-            if not any(st):
-                raise KzgError("batch failed")
+        st = _batch_status(self._lib, res, status, n)
         return out.raw[:n * 48], st
 
     def compute_blob_kzg_proof_batch(self, blobs_flat, commitments_flat, n):
@@ -280,11 +282,7 @@ class DASContext:
         status = C.create_string_buffer(max(n, 1))
         res = self._lib.eth_kzg_b200_compute_blob_kzg_proof_batch(C.c_void_p(self._ctx), C.c_uint64(n), _exact(blobs_flat, n * BYTES_PER_BLOB, "blobs"),
                                                                   _exact(commitments_flat, n * 48, "commitments"), out, status)
-        st = list(status.raw[:n])
-        if res.status != 0:
-            self._lib.eth_kzg_free_error_message(res.error_msg)
-            if not any(st):
-                raise KzgError("batch failed")
+        st = _batch_status(self._lib, res, status, n)
         return out.raw[:n * 48], st
 
     def recover_cells_and_kzg_proofs_batch(self, indices_per_blob, cells_per_blob):
@@ -298,11 +296,7 @@ class DASContext:
         op = C.create_string_buffer(max(n, 1) * CELLS_PER_EXT_BLOB * 48)
         status = C.create_string_buffer(max(n, 1))
         res = self._lib.eth_kzg_b200_recover_cells_and_kzg_proofs_batch(C.c_void_p(self._ctx), C.c_uint64(n), counts, idx, cells, oc, op, status)
-        st = list(status.raw[:n])
-        if res.status != 0:
-            self._lib.eth_kzg_free_error_message(res.error_msg)
-            if not any(st):
-                raise KzgError("batch failed")
+        st = _batch_status(self._lib, res, status, n)
         return oc.raw, op.raw, st
 
     def compute_cells_and_kzg_proofs_device(self, n, d_blobs, d_cells, d_proofs, d_status, stream=0):
