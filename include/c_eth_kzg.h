@@ -154,6 +154,24 @@ CResult eth_kzg_b200_recover_cells_and_kzg_proofs_batch(const DASContext *ctx, u
                                                         const uint64_t *cell_indices, const uint8_t *cells, uint8_t *out_cells,
                                                         uint8_t *out_proofs, uint8_t *item_status);
 
+/* verify_cell_kzg_proof_batch with a verdict per caller-defined group of openings (for example the cells of one column
+ * sidecar).  Inputs as eth_kzg_verify_cell_kzg_proof_batch (n of each), plus group_of[n] (< n_groups).  group_status[n_groups]:
+ * 0 every opening of the group verifies (also: an empty group), 1 the group's openings do not verify, 2 the group holds a
+ * malformed item (invalid commitment / proof encoding or subgroup, non-canonical cell scalar, cell index >= 128; an invalid
+ * commitment marks every group with a cell that refers to it).  *all_ok = every group is 0.  The challenge is the plain
+ * call's, so with no malformed item *all_ok equals its result.  Err only for structural faults: a group id >= n_groups,
+ * n_groups above 2^20. */
+CResult eth_kzg_b200_verify_cell_kzg_proof_batch_groups(const DASContext *ctx, uint64_t n, const uint8_t *const *commitments,
+                                                        const uint64_t *cell_indices, const uint8_t *const *cells,
+                                                        const uint8_t *const *proofs, uint64_t n_groups, const uint32_t *group_of,
+                                                        uint8_t *group_status, bool *all_ok);
+
+/* verify_blob_kzg_proof_batch with a verdict per blob: item_status[n] 0 verifies, 1 does not, 2 malformed (non-canonical
+ * blob, invalid commitment or proof).  *all_ok = every item is 0; with no malformed item it equals the plain call's result. */
+CResult eth_kzg_b200_verify_blob_kzg_proof_batch_items(const DASContext *ctx, uint64_t n, const uint8_t *const *blobs,
+                                                       const uint8_t *const *commitments, const uint8_t *const *proofs,
+                                                       uint8_t *item_status, bool *all_ok);
+
 /* CUDA device ordinal the context lives on, fixed-base window width, and bytes of HBM its tables occupy. */
 int eth_kzg_b200_context_device(const DASContext *ctx);
 int eth_kzg_b200_context_window(const DASContext *ctx);

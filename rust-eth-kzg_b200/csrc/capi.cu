@@ -323,4 +323,18 @@ CResult eth_kzg_verify_blob_kzg_proof_batch(const DASContext* ctx, uint64_t blob
     return to_c(next_cx(ctx).verify_kzg_proofs(1, blobs_length, blobs, commitments, nullptr, nullptr, proofs, verified));
 }
 
+CResult eth_kzg_b200_verify_cell_kzg_proof_batch_groups(const DASContext* ctx, uint64_t n, const uint8_t* const* commitments,
+                                                        const uint64_t* cell_indices, const uint8_t* const* cells, const uint8_t* const* proofs,
+                                                        uint64_t n_groups, const uint32_t* group_of, uint8_t* group_status, bool* all_ok) {
+    DeviceGuard guard;
+    return to_c(next_cx(ctx).verify_cell_kzg_proof_batch_groups(n, commitments, cell_indices, cells, proofs, n_groups, group_of, group_status,
+                                                                all_ok));
+}
+CResult eth_kzg_b200_verify_blob_kzg_proof_batch_items(const DASContext* ctx, uint64_t n, const uint8_t* const* blobs,
+                                                       const uint8_t* const* commitments, const uint8_t* const* proofs, uint8_t* item_status,
+                                                       bool* all_ok) {
+    DeviceGuard guard;
+    return to_c(next_cx(ctx).verify_kzg_proofs(1, n, blobs, commitments, nullptr, nullptr, proofs, all_ok, item_status));
+}
+
 }  // extern "C"

@@ -73,6 +73,19 @@ cudaError_t launch_kzg_verify_pairs(const G1Affine* commitments, const G1Affine*
                                     uint32_t* scalars, int n, cudaStream_t st);   // 4n (point, scalar) pairs, kind-major
 cudaError_t launch_poly_eval(const Fr* coeffs, const Fr* z, Fr* y, uint8_t* y_be, int B, cudaStream_t st);
 cudaError_t launch_fr_to_be(const Fr* in, uint8_t* out, int n, cudaStream_t st);
+// verdicts per group / per item: masking of malformed items, then the per-group sums of the failure path
+cudaError_t launch_cell_canonical(const uint8_t* cells, uint32_t* bad, int n, cudaStream_t st);   // bad[k] = cell k holds a value >= r
+cudaError_t launch_mask_openings(Fr* rpow, const uint32_t* stp, const uint32_t* stc, const uint32_t* row, uint32_t* col, const uint32_t* cell_bad,
+                                 G1Affine* a_p, G1Affine* a_c, uint32_t* flag, int n, int m, cudaStream_t st);
+cudaError_t launch_mask_items(Fr* rpow, const uint32_t* stb, const uint32_t* stc, const uint32_t* stp, G1Affine* a_c, G1Affine* a_p, uint32_t* flag,
+                              int n, cudaStream_t st);
+cudaError_t launch_gather_points(const G1Affine* pts, const uint32_t* idx, G1Affine* out, int n, cudaStream_t st);
+// sums[s * G + g] = sum over the CSR segment of group g of in_s (s = 0, 1, 2); groups listed in `small` get a warp, in `large` a CTA
+cudaError_t launch_group_point_sums(const G1Jac* in0, const G1Jac* in1, const G1Jac* in2, const uint32_t* order, const uint32_t* off,
+                                    const uint32_t* small, int n_small, const uint32_t* large, int n_large, G1Jac* sums, int G, cudaStream_t st);
+cudaError_t launch_group_interp_sums(const Fr* interp, const uint32_t* order, const uint32_t* off, uint32_t* out, int G, cudaStream_t st);   // [64][G] plain
+cudaError_t launch_pairing_inputs_n(const G1Jac* a, const G1Jac* b0, const G1Jac* b1, const G1Jac* b2, bool sub_b1, uint32_t* out, int n,
+                                    cudaStream_t st);
 
 
 }  // namespace ekzg

@@ -362,6 +362,155 @@ __global__ void k_fr_to_be(const Fr* __restrict__ in, uint8_t* __restrict__ out,
     fr_store_be(out + (size_t)i * 32, p);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Verdicts per group of openings / per blob (verify_cell_kzg_proof_batch_groups, verify_blob_kzg_proof_batch_items).
+// A malformed item is masked out of every sum: its power of r becomes 0 and its points the identity, so it adds nothing
+// and the other items keep their powers.  Then, only when the masked aggregate check fails, the sums are formed again per
+// group and checked group by group on the host.
+// ------------------------------------------------------------------------------------------------
+
+// bad[k] = 1 when a field element of cell k is not canonical (k_cell_interp ORs one flag for the whole batch).  A warp per cell.
+__global__ void __launch_bounds__(128)
+k_cell_canonical(const uint8_t* __restrict__ cells, uint32_t* __restrict__ bad, int n) {
+    const int k = blockIdx.x * 4 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (k >= n) return;   // (the whole warp)
+    const uint8_t* c = cells + (size_t)k * BYTES_PER_CELL;
+    const bool b = fe_plain_ge_mod(fr_load_be(c + 32 * lane)) || fe_plain_ge_mod(fr_load_be(c + 32 * (lane + 32)));
+    const bool any = __any_sync(0xffffffffu, b);
+    if (lane == 0) bad[k] = any ? 1u : 0u;
+}
+
+// Opening k is malformed when its proof, the commitment of its row or its cell is, or its cell index is >= 128:
+// flag[k] = 1, rho_k = 0, its proof point becomes the identity and its index 0 (so that no later kernel reads out of
+// bounds).  Threads below m set the invalid commitments to the identity.
+__global__ void k_mask_openings(Fr* __restrict__ rpow, const uint32_t* __restrict__ stp, const uint32_t* __restrict__ stc,
+                                const uint32_t* __restrict__ row, uint32_t* __restrict__ col, const uint32_t* __restrict__ cell_bad,
+                                G1Affine* __restrict__ a_p, G1Affine* __restrict__ a_c, uint32_t* __restrict__ flag, int n, int m) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    G1Affine id;
+    g1a_set_inf(id);
+    if (i < m && stc[i]) st_vec(&a_c[i], id);
+    if (i >= n) return;
+    const bool bad_col = col[i] >= (uint32_t)N_CELLS;
+    const bool bad = stp[i] || stc[row[i]] || cell_bad[i] || bad_col;
+    flag[i] = bad ? 1u : 0u;
+    if (bad) {
+        Fr z;
+        fe_set_zero(z);
+        st_vec(&rpow[i], z);
+        st_vec(&a_p[i], id);
+    }
+    if (bad_col) col[i] = 0;
+}
+
+// EIP-4844 item i is malformed when its blob, commitment or proof is: flag[i] = 1, r^i = 0, both points the identity
+__global__ void k_mask_items(Fr* __restrict__ rpow, const uint32_t* __restrict__ stb, const uint32_t* __restrict__ stc,
+                             const uint32_t* __restrict__ stp, G1Affine* __restrict__ a_c, G1Affine* __restrict__ a_p,
+                             uint32_t* __restrict__ flag, int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const bool bad = stb[i] || stc[i] || stp[i];
+    flag[i] = bad ? 1u : 0u;
+    if (bad) {
+        Fr z;
+        fe_set_zero(z);
+        st_vec(&rpow[i], z);
+        G1Affine id;
+        g1a_set_inf(id);
+        st_vec(&a_c[i], id);
+        st_vec(&a_p[i], id);
+    }
+}
+
+// out[k] = pts[idx[k]]  (the commitment of every opening, for a ladder per opening)
+__global__ void k_gather_points(const G1Affine* __restrict__ pts, const uint32_t* __restrict__ idx, G1Affine* __restrict__ out, int n) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    st_vec(&out[k], ld_vec(&pts[idx[k]]));
+}
+
+// Segmented point sums over a CSR layout: the items of group g are order[off[g] .. off[g + 1]).  For s = 0, 1, 2:
+// sums[s * G + g] = sum of in_s[order[j]].  TEAM threads per group: a warp for a small group (four per CTA), the whole CTA
+// for a large one; `groups[count]` lists the groups of this launch.
+template <int TEAM>
+__global__ void __launch_bounds__(128)
+k_group_point_sums(const G1Jac* __restrict__ in0, const G1Jac* __restrict__ in1, const G1Jac* __restrict__ in2,
+                   const uint32_t* __restrict__ order, const uint32_t* __restrict__ off, const uint32_t* __restrict__ groups, int count,
+                   G1Jac* __restrict__ sums, int G) {
+    __shared__ G1Jac sm[128];
+    const int team = blockIdx.x * (128 / TEAM) + threadIdx.x / TEAM, lane = threadIdx.x % TEAM;
+    const bool live = team < count;
+    const int g = live ? (int)groups[team] : 0;
+    const int lo = live ? (int)off[g] : 0, hi = live ? (int)off[g + 1] : 0;
+#pragma unroll 1
+    for (int s = 0; s < 3; s++) {
+        const G1Jac* in = s == 0 ? in0 : (s == 1 ? in1 : in2);
+        G1Jac acc;
+        jac_set_inf(acc);
+        for (int j = lo + lane; j < hi; j += TEAM) {
+            G1Jac q = ld_vec(&in[order[j]]);
+            jac_add(acc, q);
+        }
+        sm[threadIdx.x] = acc;
+        __syncthreads();
+        for (int w = TEAM / 2; w >= 1; w >>= 1) {
+            if (lane < w) {
+                G1Jac a = sm[threadIdx.x];
+                jac_add(a, sm[threadIdx.x + w]);
+                sm[threadIdx.x] = a;
+            }
+            __syncthreads();
+        }
+        if (live && lane == 0) st_vec(&sums[(size_t)s * G + g], sm[threadIdx.x]);
+        __syncthreads();
+    }
+}
+
+// out[(t * G + g) * 8] = sum over the items of group g of interp[k][t], as plain integers.  t-major ([64][G]): the layout
+// in which the fixed-base MSM reads the scalars of G "blobs" (for G = 1 that of k_interp_column_sum).  A CTA per group,
+// four lanes per coefficient.
+__global__ void __launch_bounds__(256)
+k_group_interp_sums(const Fr* __restrict__ interp, const uint32_t* __restrict__ order, const uint32_t* __restrict__ off,
+                    uint32_t* __restrict__ out, int G) {
+    __shared__ Fr sm[256];
+    const int g = blockIdx.x, t = threadIdx.x & 63, q = threadIdx.x >> 6;
+    Fr acc;
+    fe_set_zero(acc);
+    for (int j = (int)off[g] + q; j < (int)off[g + 1]; j += 4) {
+        Fr v = ld_vec(&interp[(size_t)order[j] * 64 + t]);
+        fe_add(acc, acc, v);
+    }
+    sm[threadIdx.x] = acc;
+    __syncthreads();
+    if (q != 0) return;
+    for (int r = 1; r < 4; r++) {
+        Fr b = sm[threadIdx.x + 64 * r];
+        fe_add(acc, acc, b);
+    }
+    store_plain(out + ((size_t)t * G + g) * 8, acc);
+}
+
+// n pairing checks in the layout of k_pairing_inputs, one thread each: P_i = a[i], Q_i = b0[i] + b1[i] + b2[i], or
+// b0[i] - b1[i] + b2[i] with sub_b1
+__global__ void k_pairing_inputs_n(const G1Jac* __restrict__ a, const G1Jac* __restrict__ b0, const G1Jac* __restrict__ b1,
+                                   const G1Jac* __restrict__ b2, bool sub_b1, uint32_t* __restrict__ out, int n) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    G1Jac pt[2];
+    pt[0] = ld_vec(&a[i]);
+    pt[1] = ld_vec(&b0[i]);
+    G1Jac q = ld_vec(&b1[i]);
+    if (sub_b1) jac_neg(q, q);
+    jac_add(pt[1], q);
+    q = ld_vec(&b2[i]);
+    jac_add(pt[1], q);
+    for (int h = 0; h < 2; h++) {
+        uint32_t* o = out + (size_t)PAIRING_INPUT_WORDS * (2 * i + h);
+        for (int l = 0; l < 12; l++) { o[l] = pt[h].x.v[l]; o[12 + l] = pt[h].y.v[l]; o[24 + l] = pt[h].z.v[l]; }
+        o[36] = jac_is_inf(pt[h]) ? 1u : 0u;
+    }
+}
+
 
 cudaError_t launch_powers_from_hash(const uint8_t* hash, Fr* rpow, int n, cudaStream_t st) {
     k_powers_from_hash<<<(n + 127) / 128, 128, 0, st>>>(hash, rpow, n);
@@ -434,6 +583,51 @@ cudaError_t launch_poly_eval(const Fr* coeffs, const Fr* z, Fr* y, uint8_t* y_be
 }
 cudaError_t launch_fr_to_be(const Fr* in, uint8_t* out, int n, cudaStream_t st) {
     k_fr_to_be<<<(n + 127) / 128, 128, 0, st>>>(in, out, n);
+    EKZG_LAUNCH_CHECK();
+    return cudaSuccess;
+}
+cudaError_t launch_cell_canonical(const uint8_t* cells, uint32_t* bad, int n, cudaStream_t st) {
+    k_cell_canonical<<<(n + 3) / 4, 128, 0, st>>>(cells, bad, n);
+    EKZG_LAUNCH_CHECK();
+    return cudaSuccess;
+}
+cudaError_t launch_mask_openings(Fr* rpow, const uint32_t* stp, const uint32_t* stc, const uint32_t* row, uint32_t* col, const uint32_t* cell_bad,
+                                 G1Affine* a_p, G1Affine* a_c, uint32_t* flag, int n, int m, cudaStream_t st) {
+    k_mask_openings<<<(std::max(n, m) + 127) / 128, 128, 0, st>>>(rpow, stp, stc, row, col, cell_bad, a_p, a_c, flag, n, m);
+    EKZG_LAUNCH_CHECK();
+    return cudaSuccess;
+}
+cudaError_t launch_mask_items(Fr* rpow, const uint32_t* stb, const uint32_t* stc, const uint32_t* stp, G1Affine* a_c, G1Affine* a_p, uint32_t* flag,
+                              int n, cudaStream_t st) {
+    k_mask_items<<<(n + 127) / 128, 128, 0, st>>>(rpow, stb, stc, stp, a_c, a_p, flag, n);
+    EKZG_LAUNCH_CHECK();
+    return cudaSuccess;
+}
+cudaError_t launch_gather_points(const G1Affine* pts, const uint32_t* idx, G1Affine* out, int n, cudaStream_t st) {
+    k_gather_points<<<(n + 127) / 128, 128, 0, st>>>(pts, idx, out, n);
+    EKZG_LAUNCH_CHECK();
+    return cudaSuccess;
+}
+cudaError_t launch_group_point_sums(const G1Jac* in0, const G1Jac* in1, const G1Jac* in2, const uint32_t* order, const uint32_t* off,
+                                    const uint32_t* small, int n_small, const uint32_t* large, int n_large, G1Jac* sums, int G, cudaStream_t st) {
+    if (n_small) {
+        k_group_point_sums<32><<<(n_small + 3) / 4, 128, 0, st>>>(in0, in1, in2, order, off, small, n_small, sums, G);
+        EKZG_LAUNCH_CHECK();
+    }
+    if (n_large) {
+        k_group_point_sums<128><<<n_large, 128, 0, st>>>(in0, in1, in2, order, off, large, n_large, sums, G);
+        EKZG_LAUNCH_CHECK();
+    }
+    return cudaSuccess;
+}
+cudaError_t launch_group_interp_sums(const Fr* interp, const uint32_t* order, const uint32_t* off, uint32_t* out, int G, cudaStream_t st) {
+    k_group_interp_sums<<<G, 256, 0, st>>>(interp, order, off, out, G);
+    EKZG_LAUNCH_CHECK();
+    return cudaSuccess;
+}
+cudaError_t launch_pairing_inputs_n(const G1Jac* a, const G1Jac* b0, const G1Jac* b1, const G1Jac* b2, bool sub_b1, uint32_t* out, int n,
+                                    cudaStream_t st) {
+    k_pairing_inputs_n<<<(n + 63) / 64, 64, 0, st>>>(a, b0, b1, b2, sub_b1, out, n);
     EKZG_LAUNCH_CHECK();
     return cudaSuccess;
 }

@@ -37,6 +37,14 @@ enum ItemStatus : uint8_t {
     ITEM_BAD_INDICES = 3,     // recovery: cell indices out of range, not ascending, too few or too many
     ITEM_BAD_DEGREE = 4,      // recovery: the recovered polynomial has degree >= 4096
 };
+// Verdicts of the verifiers that answer per group of openings / per blob (group_status / item_status of the C ABI: the
+// values are fixed).
+enum Verdict : uint8_t {
+    VERDICT_OK = 0,          // verifies (an empty group too)
+    VERDICT_FAILS = 1,       // well-formed, does not verify
+    VERDICT_MALFORMED = 2,   // holds an invalid point encoding / subgroup, a non-canonical scalar or a cell index >= 128
+};
+constexpr uint64_t MAX_VERIFY_GROUPS = 1u << 20;
 // The error text of an item with status `code`: `cells` -- its inputs were cells (recovery), not a blob; `z` -- its second
 // input was an evaluation point, not a commitment.
 const char* item_status_text(uint8_t code, bool cells, bool z);
@@ -161,9 +169,15 @@ public:
     Status verify_cell_kzg_proof_batch(uint64_t n_commitments, const uint8_t* const* commitments, uint64_t n_indices,
                                        const uint64_t* cell_indices, uint64_t n_cells, const uint8_t* const* cells, uint64_t n_proofs,
                                        const uint8_t* const* proofs, bool* verified) const;
-    // mode 0: verify_kzg_proof items (commitment, z, y, proof); mode 1: verify_blob_kzg_proof(_batch) items (blob, commitment, proof)
+    // The same check with a Verdict per caller-defined group of openings: group_of[n] < n_groups, group_status[n_groups].
+    // *all_ok = every group is VERDICT_OK.  Err only for a group id >= n_groups or n_groups > MAX_VERIFY_GROUPS.
+    Status verify_cell_kzg_proof_batch_groups(uint64_t n, const uint8_t* const* commitments, const uint64_t* cell_indices,
+                                              const uint8_t* const* cells, const uint8_t* const* proofs, uint64_t n_groups,
+                                              const uint32_t* group_of, uint8_t* group_status, bool* all_ok) const;
+    // mode 0: verify_kzg_proof items (commitment, z, y, proof); mode 1: verify_blob_kzg_proof(_batch) items (blob, commitment, proof).
+    // item_status (mode 1 only, optional): a Verdict per item instead of Err for malformed items; *verified = all are VERDICT_OK.
     Status verify_kzg_proofs(int mode, uint64_t n, const uint8_t* const* blobs, const uint8_t* const* commitments, const uint8_t* z32,
-                             const uint8_t* y32, const uint8_t* const* proofs, bool* verified) const;
+                             const uint8_t* y32, const uint8_t* const* proofs, bool* verified, uint8_t* item_status = nullptr) const;
 
     // workspace pool (calls are re-entrant: concurrent callers each borrow their own workspaces)
     Workspace* acquire(int min_capacity, bool with_io) const;
@@ -188,6 +202,14 @@ private:
     Status run_4844(Mode4844 mode, uint64_t n, const uint8_t* blobs, const uint8_t* aux_in, uint8_t* out48, uint8_t* out_y32,
                     uint8_t* item_status) const;
     Context() = default;
+    // both cell verifiers: n openings, lengths and (plain call) indices already checked; `groups` == nullptr: the plain call
+    struct GroupVerdicts {
+        const uint32_t* group_of;
+        uint64_t n_groups;
+        uint8_t* status;
+    };
+    Status verify_cells(uint64_t n, const uint8_t* const* commitments, const uint64_t* cell_indices, const uint8_t* const* cells,
+                        const uint8_t* const* proofs, const GroupVerdicts* groups, bool* verified) const;
     // proofs of n blobs from ws.d_coeffs, asynchronous on `stream`: by the direct route when proof_route() picks it
     // (never with stage_events), else FK20 = fk20_msm of all n blobs, then fk20_ntt_compress
     Status fk20_from_coeffs_device(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream,

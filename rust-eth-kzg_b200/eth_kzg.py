@@ -69,6 +69,9 @@ def load_library():
                  "eth_kzg_b200_recover_cells_and_kzg_proofs_batch", "eth_kzg_b200_blob_to_kzg_commitment_batch", "eth_kzg_b200_compute_blob_kzg_proof_batch",
                  "eth_kzg_b200_das_context_new_from_json", "eth_kzg_b200_debug_parse_trusted_setup_json", "eth_kzg_b200_debug_g2_keys"):
         getattr(lib, name).restype = _CResult
+    for name in ("eth_kzg_b200_verify_cell_kzg_proof_batch_groups", "eth_kzg_b200_verify_blob_kzg_proof_batch_items"):
+        if hasattr(lib, name):   # (an EKZG_LIB build from before these entry points lacks them)
+            getattr(lib, name).restype = _CResult
     _lib = lib
     return lib
 
@@ -221,6 +224,33 @@ class DASContext:
         del k1, k2, k3
         return bool(ok.value)
 
+    def verify_cell_kzg_proof_batch_groups(self, commitments, cell_indices, cells, proofs, groups, n_groups=None):
+        """verify_cell_kzg_proof_batch with a verdict per caller-defined group: opening k belongs to group groups[k]
+        (< n_groups, default max(groups) + 1).  -> (all_ok, [status per group]): 0 verifies (also an empty group), 1 does not,
+        2 holds a malformed item (invalid commitment / proof, non-canonical cell, cell index >= 128).  Raises KzgError only
+        for structural faults: lengths that differ, a group id >= n_groups, n_groups above 2^20."""
+        n = len(commitments)
+        if not (n == len(cell_indices) == len(cells) == len(proofs) == len(groups)):
+            raise KzgError("Verifier(BatchVerificationInputsMustHaveSameLength)")
+        if n_groups is None:
+            n_groups = max(groups) + 1 if n else 0
+        if min(groups, default=0) < 0 or max(groups, default=0) >= 1 << 32:
+            raise KzgError("group id out of range")
+        commitments = [_exact(c, 48, "commitment") for c in commitments]
+        cells = [_exact(c, BYTES_PER_CELL, "cell") for c in cells]
+        proofs = [_exact(p, 48, "proof") for p in proofs]
+        ca, k1 = _ptr_array(commitments)
+        cl, k2 = _ptr_array(cells)
+        pa, k3 = _ptr_array(proofs)
+        idx = (C.c_uint64 * max(n, 1))(*cell_indices)
+        grp = (C.c_uint32 * max(n, 1))(*groups)
+        status = C.create_string_buffer(max(n_groups, 1)) if n_groups <= 1 << 20 else None
+        ok = C.c_bool(False)
+        _check(self._lib, self._lib.eth_kzg_b200_verify_cell_kzg_proof_batch_groups(
+            C.c_void_p(self._ctx), C.c_uint64(n), ca, idx, cl, pa, C.c_uint64(n_groups), grp, status, C.byref(ok)))
+        del k1, k2, k3
+        return bool(ok.value), list(status.raw[:n_groups])
+
     # ---- EIP-4844 methods re-exported on DASContext (crates/eip7594/src/eip4844_methods.rs:13-77) ----
     def compute_kzg_proof(self, blob, z):
         proof, y = C.create_string_buffer(48), C.create_string_buffer(32)
@@ -257,6 +287,25 @@ class DASContext:
             C.c_void_p(self._ctx), C.c_uint64(len(blobs)), ba, C.c_uint64(len(commitments)), ca, C.c_uint64(len(proofs)), pa, C.byref(ok)))
         del k1, k2, k3
         return bool(ok.value)
+
+    def verify_blob_kzg_proof_batch_items(self, blobs, commitments, proofs):
+        """verify_blob_kzg_proof_batch with a verdict per blob -> (all_ok, [status]): 0 verifies, 1 does not, 2 malformed
+        (non-canonical blob, invalid commitment or proof).  Raises KzgError only when the lengths differ."""
+        n = len(blobs)
+        if not (n == len(commitments) == len(proofs)):
+            raise KzgError("Verifier(BatchVerificationInputsMustHaveSameLength)")
+        blobs = [_exact(b, BYTES_PER_BLOB, "blob") for b in blobs]
+        commitments = [_exact(c, 48, "commitment") for c in commitments]
+        proofs = [_exact(p, 48, "proof") for p in proofs]
+        ba, k1 = _ptr_array(blobs)
+        ca, k2 = _ptr_array(commitments)
+        pa, k3 = _ptr_array(proofs)
+        status = C.create_string_buffer(max(n, 1))
+        ok = C.c_bool(False)
+        _check(self._lib, self._lib.eth_kzg_b200_verify_blob_kzg_proof_batch_items(C.c_void_p(self._ctx), C.c_uint64(n), ba, ca, pa, status,
+                                                                                   C.byref(ok)))
+        del k1, k2, k3
+        return bool(ok.value), list(status.raw[:n])
 
     # ---- additive batch / device entry points --------------------------------------------------
     def compute_cells_and_kzg_proofs_batch(self, blobs_flat, n, want_proofs=True):

@@ -6,7 +6,9 @@ kernels when their files are equal.
   EKZG_LIB=path/to/libc_eth_kzg_b200.so python tools/launch_sequence.py --out launches.json
 
 Calls: compute_cells_and_kzg_proofs batch (1, 2, 8, 33, 1024 blobs), the device entry point (1, 1024), recovery batch
-(1, 40), blob_to_kzg_commitment batch and compute_blob_kzg_proof batch (1, 40) and compute_kzg_proof (1 call, 40 calls).
+(1, 40), blob_to_kzg_commitment batch and compute_blob_kzg_proof batch (1, 40), compute_kzg_proof (1 call, 40 calls), the
+verifiers verify_cell_kzg_proof_batch (128 and 16 384 openings) and verify_blob_kzg_proof_batch (1, 20 blobs), and, where the
+build has them, the grouped cell verifier and the per-blob verifier on the same inputs (honest, and with one bad item).
 Each call runs once before it is counted, so first-use allocations are not part of it."""
 import argparse
 import ctypes as C
@@ -93,6 +95,30 @@ def main():
         res["commitment_batch_%d" % n] = record(lib, lambda n=n: ctx.blob_to_kzg_commitment_batch(flat[:n * 131072], n))
         res["blob_proof_batch_%d" % n] = record(lib, lambda n=n: ctx.compute_blob_kzg_proof_batch(flat[:n * 131072], comm[:n * 48], n))
         res["kzg_proof_x%d" % n] = record(lib, lambda n=n: [ctx.compute_kzg_proof(flat[i * 131072:(i + 1) * 131072], z) for i in range(n)])
+
+    nb = 128
+    cms, _ = ctx.blob_to_kzg_commitment_batch(flat[:nb * 131072], nb)
+    cells, proofs, _ = ctx.compute_cells_and_kzg_proofs_batch(flat[:nb * 131072], nb)
+    C = [cms[48 * (k // 128):48 * (k // 128) + 48] for k in range(nb * 128)]
+    I = [k % 128 for k in range(nb * 128)]
+    CL = [cells[k * 2048:(k + 1) * 2048] for k in range(nb * 128)]
+    PR = [proofs[k * 48:(k + 1) * 48] for k in range(nb * 128)]
+    bad = list(CL)
+    bad[100] = bad[100][:31] + bytes([bad[100][31] ^ 1]) + bad[100][32:]
+    bl = [flat[i * 131072:(i + 1) * 131072] for i in range(20)]
+    bp, _ = ctx.compute_blob_kzg_proof_batch(flat[:20 * 131072], comm[:20 * 48], 20)
+    bcl = [comm[48 * i:48 * i + 48] for i in range(20)]
+    bpl = [bp[48 * i:48 * i + 48] for i in range(20)]
+    for n in (128, 16384):
+        res["verify_cells_%d" % n] = record(lib, lambda n=n: ctx.verify_cell_kzg_proof_batch(C[:n], I[:n], CL[:n], PR[:n]))
+    for n in (1, 20):
+        res["verify_blobs_%d" % n] = record(lib, lambda n=n: ctx.verify_blob_kzg_proof_batch(bl[:n], bcl[:n], bpl[:n]))
+    if hasattr(lib, "eth_kzg_b200_verify_cell_kzg_proof_batch_groups"):
+        for name, cl in (("honest", CL), ("one_bad", bad)):
+            res["verify_cells_groups_16384_%s" % name] = record(lib, lambda cl=cl: ctx.verify_cell_kzg_proof_batch_groups(C, I, cl, PR, I))
+        swapped = bpl[:1] + [bpl[2], bpl[1]] + bpl[3:]
+        for name, pl in (("honest", bpl), ("one_bad", swapped)):
+            res["verify_blobs_items_20_%s" % name] = record(lib, lambda pl=pl: ctx.verify_blob_kzg_proof_batch_items(bl, bcl, pl))
     ctx.close()
 
     with open(args.out, "w") as f:
