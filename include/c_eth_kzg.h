@@ -172,6 +172,25 @@ CResult eth_kzg_b200_verify_blob_kzg_proof_batch_items(const DASContext *ctx, ui
                                                        const uint8_t *const *commitments, const uint8_t *const *proofs,
                                                        uint8_t *item_status, bool *all_ok);
 
+/* The cell proofs of whole blobs, as an EIP-7594 blob transaction carries them (blob, commitment, 128 cell proofs), checked by
+ * recomputing each blob's commitment and proofs on the device and comparing bytes: no cells leave the device, no transcript is
+ * hashed, no randomness.  Contiguous HOST buffers: blobs n*131072 B, commitments n*48 B, proofs n*128*48 B in cell order
+ * (pinned memory is DMA'd as it is, pageable memory staged).
+ *   item_status[n]: 2 malformed (non-canonical blob, or the commitment or any proof is not a valid compressed G1 point in the
+ *     subgroup), else 1 if the commitment or any proof differs from the blob's own, else 0.  Values and precedence as
+ *     eth_kzg_b200_verify_blob_kzg_proof_batch_items.
+ *   cell_status[n*128] (may be NULL): 0 proof k is the proof of cell k of the blob, 1 a valid point but not that proof, 2 not a
+ *     valid encoding; all 2 for a non-canonical blob.  It does not depend on the commitment: it states a fact about the proof
+ *     and the blob only.
+ *   *all_ok = every item is 0.  Err only for allocation or CUDA failures; n = 0 gives Ok with *all_ok = true.
+ * Soundness: where the commitment is the blob's, a cell proof is accepted by the reference verifier iff it equals the one
+ * recomputed here (the single-opening equation has exactly one solution).  Where it is not, the reference accepts all 128
+ * openings only if KZG binding breaks; single openings it may accept, which this call reports as item 1.  The call is
+ * deterministic; the reference's batch check errs with probability <= n/|Fr|. */
+CResult eth_kzg_b200_verify_blob_cell_proofs_batch(const DASContext *ctx, uint64_t n, const uint8_t *blobs,
+                                                   const uint8_t *commitments, const uint8_t *proofs, uint8_t *item_status,
+                                                   uint8_t *cell_status, bool *all_ok);
+
 /* CUDA device ordinal the context lives on, fixed-base window width, and bytes of HBM its tables occupy. */
 int eth_kzg_b200_context_device(const DASContext *ctx);
 int eth_kzg_b200_context_window(const DASContext *ctx);

@@ -336,5 +336,10 @@ CResult eth_kzg_b200_verify_blob_kzg_proof_batch_items(const DASContext* ctx, ui
     DeviceGuard guard;
     return to_c(next_cx(ctx).verify_kzg_proofs(1, n, blobs, commitments, nullptr, nullptr, proofs, all_ok, item_status));
 }
+CResult eth_kzg_b200_verify_blob_cell_proofs_batch(const DASContext* ctx, uint64_t n, const uint8_t* blobs, const uint8_t* commitments,
+                                                   const uint8_t* proofs, uint8_t* item_status, uint8_t* cell_status, bool* all_ok) {
+    DeviceGuard guard;
+    return to_c(ds(ctx).verify_blob_cell_proofs_batch(n, blobs, commitments, proofs, item_status, cell_status, all_ok));
+}
 
 }  // extern "C"

@@ -86,6 +86,12 @@ cudaError_t launch_group_point_sums(const G1Jac* in0, const G1Jac* in1, const G1
 cudaError_t launch_group_interp_sums(const Fr* interp, const uint32_t* order, const uint32_t* off, uint32_t* out, int G, cudaStream_t st);   // [64][G] plain
 cudaError_t launch_pairing_inputs_n(const G1Jac* a, const G1Jac* b0, const G1Jac* b1, const G1Jac* b2, bool sub_b1, uint32_t* out, int n,
                                     cudaStream_t st);
+// verify_blob_cell_proofs_batch: byte comparison of B blobs' recomputed proofs (B x 128 x 48 B) and commitments (B x 48 B) with the
+// supplied ones; cell_mm[B][128]: 0 equal, 1 differs, 2 blob_status[b] != 0 (non-canonical blob); blob_mm[B]: BLOB_MM_* bits
+enum : uint8_t { BLOB_MM_PROOF = 1, BLOB_MM_COMMITMENT = 2, BLOB_MM_NON_CANONICAL = 4 };
+cudaError_t launch_compare_blob_proofs(const uint8_t* computed_proofs, const uint8_t* given_proofs, const uint8_t* computed_c48,
+                                       const uint8_t* given_c48, const uint32_t* blob_status, uint8_t* cell_mm, uint8_t* blob_mm, int B,
+                                       cudaStream_t st);
 
 
 }  // namespace ekzg

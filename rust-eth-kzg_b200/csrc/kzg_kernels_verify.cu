@@ -511,6 +511,36 @@ __global__ void k_pairing_inputs_n(const G1Jac* __restrict__ a, const G1Jac* __r
     }
 }
 
+// verify_blob_cell_proofs_batch: the recomputed compressed proofs and commitment of each blob against the supplied bytes.  One
+// CTA of 128 threads per blob, thread k on cell k (three 16-byte loads per side; 48-byte records at 16-byte aligned bases).
+// cell_mm[b * 128 + k]: 0 equal, 1 differs, 2 the blob is non-canonical (K1's status; then the computed bytes mean nothing).
+// blob_mm[b]: BLOB_MM_* bits.
+__global__ void __launch_bounds__(128)
+k_compare_blob_proofs(const uint8_t* __restrict__ computed_proofs, const uint8_t* __restrict__ given_proofs,
+                      const uint8_t* __restrict__ computed_c48, const uint8_t* __restrict__ given_c48, const uint32_t* __restrict__ blob_status,
+                      uint8_t* __restrict__ cell_mm, uint8_t* __restrict__ blob_mm) {
+    const int b = blockIdx.x, k = threadIdx.x;
+    const bool non_canonical = blob_status[b] != 0;
+    const size_t at = ((size_t)b * N_CELLS + k) * BYTES_PER_G1 / 16;
+    const uint4* p = reinterpret_cast<const uint4*>(computed_proofs) + at;
+    const uint4* q = reinterpret_cast<const uint4*>(given_proofs) + at;
+    bool differs = false;
+#pragma unroll
+    for (int i = 0; i < 3; i++) {
+        const uint4 x = p[i], y = q[i];
+        differs |= x.x != y.x || x.y != y.y || x.z != y.z || x.w != y.w;
+    }
+    cell_mm[(size_t)b * N_CELLS + k] = non_canonical ? 2 : (differs ? 1 : 0);
+    bool c_differs = false;
+    if (k < 3) {
+        const uint4 x = reinterpret_cast<const uint4*>(computed_c48)[(size_t)b * 3 + k], y = reinterpret_cast<const uint4*>(given_c48)[(size_t)b * 3 + k];
+        c_differs = x.x != y.x || x.y != y.y || x.z != y.z || x.w != y.w;
+    }
+    const int any_proof = __syncthreads_or(differs), any_c = __syncthreads_or(c_differs);
+    if (k == 0)
+        blob_mm[b] = (uint8_t)((any_proof ? BLOB_MM_PROOF : 0) | (any_c ? BLOB_MM_COMMITMENT : 0) | (non_canonical ? BLOB_MM_NON_CANONICAL : 0));
+}
+
 
 cudaError_t launch_powers_from_hash(const uint8_t* hash, Fr* rpow, int n, cudaStream_t st) {
     k_powers_from_hash<<<(n + 127) / 128, 128, 0, st>>>(hash, rpow, n);
@@ -628,6 +658,13 @@ cudaError_t launch_group_interp_sums(const Fr* interp, const uint32_t* order, co
 cudaError_t launch_pairing_inputs_n(const G1Jac* a, const G1Jac* b0, const G1Jac* b1, const G1Jac* b2, bool sub_b1, uint32_t* out, int n,
                                     cudaStream_t st) {
     k_pairing_inputs_n<<<(n + 63) / 64, 64, 0, st>>>(a, b0, b1, b2, sub_b1, out, n);
+    EKZG_LAUNCH_CHECK();
+    return cudaSuccess;
+}
+cudaError_t launch_compare_blob_proofs(const uint8_t* computed_proofs, const uint8_t* given_proofs, const uint8_t* computed_c48,
+                                       const uint8_t* given_c48, const uint32_t* blob_status, uint8_t* cell_mm, uint8_t* blob_mm, int B,
+                                       cudaStream_t st) {
+    k_compare_blob_proofs<<<B, N_CELLS, 0, st>>>(computed_proofs, given_proofs, computed_c48, given_c48, blob_status, cell_mm, blob_mm);
     EKZG_LAUNCH_CHECK();
     return cudaSuccess;
 }

@@ -1,5 +1,6 @@
 // One DASContext over several GPUs (see kzg_multi.h).
 #include "kzg_multi.h"
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -143,6 +144,18 @@ Status DeviceSet::recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t*
                                                     out_cells + lo * CELLS_PER_BLOB, out_proofs + lo * PROOFS_PER_BLOB,
                                                     item_status ? item_status + lo : nullptr);
     });
+}
+
+Status DeviceSet::verify_blob_cell_proofs_batch(uint64_t n, const uint8_t* blobs, const uint8_t* commitments, const uint8_t* proofs,
+                                                uint8_t* item_status, uint8_t* cell_status, bool* all_ok) const {
+    *all_ok = false;
+    EKZG_TRY(fan_out(n, [&](const Context& c, uint64_t lo, uint64_t cnt) {
+        bool shard_ok = false;   // unused: each shard's verdict covers only its items; the batch verdict is formed from item_status below
+        return c.verify_blob_cell_proofs_batch(cnt, blobs + lo * BYTES_PER_BLOB, commitments + lo * BYTES_PER_G1, proofs + lo * PROOFS_PER_BLOB,
+                                               item_status + lo, cell_status ? cell_status + lo * N_CELLS : nullptr, &shard_ok);
+    }));
+    *all_ok = std::all_of(item_status, item_status + n, [](uint8_t s) { return s == VERDICT_OK; });
+    return Status::Ok();
 }
 
 uint64_t DeviceSet::table_bytes() const {

@@ -42,6 +42,8 @@ public:
                                         uint8_t* item_status) const;
     Status recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
                                               uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const;
+    Status verify_blob_cell_proofs_batch(uint64_t n, const uint8_t* blobs, const uint8_t* commitments, const uint8_t* proofs,
+                                         uint8_t* item_status, uint8_t* cell_status, bool* all_ok) const;
 
     uint64_t table_bytes() const;
 

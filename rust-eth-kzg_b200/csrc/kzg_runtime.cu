@@ -161,12 +161,41 @@ void Workspace::free_recover_buffers() {
     d_rcells = nullptr; h_rcells = nullptr; d_slotmap = nullptr; h_slotmap = nullptr; d_ze = nullptr; d_czinv = nullptr;
 }
 
+Status Workspace::ensure_verify_buffers(int blobs) {
+    if (verify_capacity >= blobs) return Status::Ok();
+    free_verify_buffers();   // (idle: the workspace is borrowed by one call at a time, and its last user synchronised it)
+    auto all = [&]() -> Status {
+        EKZG_CUDA(cudaMalloc(&d_given_proofs, (size_t)blobs * PROOFS_PER_BLOB));
+        EKZG_CUDA(cudaMalloc(&d_cell_mm, (size_t)blobs * (N_CELLS + 1)));
+        EKZG_CUDA(cudaMallocHost(&h_cell_mm, (size_t)blobs * (N_CELLS + 1)));
+        EKZG_CUDA(cudaMallocHost(&h_c48, (size_t)blobs * BYTES_PER_G1));
+        return Status::Ok();
+    };
+    Status s = all();
+    if (!s.ok) {   // all or none, as the recovery buffers
+        free_verify_buffers();
+        cudaGetLastError();
+        return s;
+    }
+    d_blob_mm = d_cell_mm + (size_t)blobs * N_CELLS;
+    h_blob_mm = h_cell_mm + (size_t)blobs * N_CELLS;
+    verify_capacity = blobs;
+    return Status::Ok();
+}
+
+void Workspace::free_verify_buffers() {
+    cudaFree(d_given_proofs); cudaFree(d_cell_mm); cudaFreeHost(h_cell_mm); cudaFreeHost(h_c48);
+    d_given_proofs = nullptr; d_cell_mm = nullptr; d_blob_mm = nullptr; h_cell_mm = nullptr; h_blob_mm = nullptr; h_c48 = nullptr;
+    verify_capacity = 0;
+}
+
 void Workspace::synchronize() const {
     for (cudaStream_t s : {stream, copy_stream, in_stream, aux_stream}) cudaStreamSynchronize(s);
 }
 
 void Workspace::release() {
     free_recover_buffers();
+    free_verify_buffers();
     cudaFree(d_c48); cudaFree(d_z32); cudaFree(d_out48); cudaFree(d_z); cudaFree(d_aff); cudaFree(d_status2);
     cudaFree(d_blobs); cudaFree(d_coeffs); cudaFree(d_cells); cudaFree(d_scalars); cudaFree(d_pts); cudaFree(d_queue); cudaFree(d_ntt_scratch); cudaFree(d_msm_scratch); cudaFree(d_proofs); cudaFree(d_status);
     cudaFreeHost(h_blobs); cudaFreeHost(h_cells); cudaFreeHost(h_proofs); cudaFreeHost(h_status);
@@ -484,10 +513,20 @@ Status Context::proofs_direct_device(Workspace& ws, int n, uint8_t* d_proofs, cu
     const int Bv = N_CELLS * n;
     if (Bv > ws.capacity) return Status::Error("workspace too small for the direct proof path");
     EKZG_CUDA(launch_coset_quotients(ws.d_coeffs, ws.d_scalars, T_, n, stream));
-    EKZG_CUDA(launch_fixed_msm(ws.d_scalars, ws.d_pts, T_.srs, N_BLOB / FK20_POINTS, Bv, stream, 0, -1, ws.d_msm_scratch));
-    EKZG_CUDA(launch_sum_positions(ws.d_pts, Bv, N_BLOB / FK20_POINTS, 2, stream));
-    EKZG_CUDA(launch_g1_compress(ws.d_pts, d_proofs, 1, Bv, stream));
+    return srs_msm_compress(ws, Bv, d_proofs, stream);
+}
+
+// fixed-base MSM (64 partial sums per item) -> tree sum -> compression
+Status Context::srs_msm_compress(Workspace& ws, int B, uint8_t* d_out, cudaStream_t stream) const {
+    EKZG_CUDA(launch_fixed_msm(ws.d_scalars, ws.d_pts, T_.srs, N_BLOB / FK20_POINTS, B, stream, 0, -1, ws.d_msm_scratch));
+    EKZG_CUDA(launch_sum_positions(ws.d_pts, B, N_BLOB / FK20_POINTS, 2, stream));
+    EKZG_CUDA(launch_g1_compress(ws.d_pts, d_out, 1, B, stream));
     return Status::Ok();
+}
+
+Status Context::commit_device(Workspace& ws, int n, uint8_t* d_out48, cudaStream_t stream) const {
+    EKZG_CUDA(launch_coeffs_to_scalars(ws.d_coeffs, ws.d_scalars, n, stream));
+    return srs_msm_compress(ws, n, d_out48, stream);
 }
 
 Status Context::fk20_msm(Workspace& ws, int n, int o, int c, cudaStream_t stream, std::vector<cudaEvent_t>* ev) const {
@@ -540,23 +579,31 @@ static bool host_range_is_pinned(const void* p) {
     return a.type == cudaMemoryTypeHost;
 }
 
-// blobs [o, o + cnt) of the chunk at `chunk` -> the same slots of ws.d_blobs, on `st`.  Pinned caller memory is DMA'd as it
-// is; pageable memory is copied into the same slots of the pinned staging buffer in slices, each slice's H2D running while
-// the host copies the next one.
-static Status upload_blobs(Workspace& ws, const uint8_t* chunk, int o, int cnt, bool src_pinned, cudaStream_t st) {
-    const size_t off = (size_t)o * BYTES_PER_BLOB;
+// items [o, o + cnt) of `item` bytes each of the chunk at `chunk` -> the same slots of `dev`, on `st`.  Pinned caller memory is
+// DMA'd as it is; pageable memory is copied into the same slots of the pinned staging buffer `stage` in slices of 8 MiB (64
+// blobs), each slice's H2D running while the host copies the next one.
+static Status upload(uint8_t* dev, uint8_t* stage, const uint8_t* chunk, size_t item, int o, int cnt, bool src_pinned, cudaStream_t st) {
+    const size_t off = (size_t)o * item;
     if (src_pinned) {
-        EKZG_CUDA(cudaMemcpyAsync(ws.d_blobs + off, chunk + off, (size_t)cnt * BYTES_PER_BLOB, cudaMemcpyHostToDevice, st));
+        EKZG_CUDA(cudaMemcpyAsync(dev + off, chunk + off, (size_t)cnt * item, cudaMemcpyHostToDevice, st));
         return Status::Ok();
     }
-    const int slice = 64;
+    const int slice = (int)std::max<size_t>(1, (size_t)64 * BYTES_PER_BLOB / item);
     for (int i = 0; i < cnt; i += slice) {
-        const size_t at = off + (size_t)i * BYTES_PER_BLOB, bytes = (size_t)std::min(slice, cnt - i) * BYTES_PER_BLOB;
-        memcpy(ws.h_blobs + at, chunk + at, bytes);
-        EKZG_CUDA(cudaMemcpyAsync(ws.d_blobs + at, ws.h_blobs + at, bytes, cudaMemcpyHostToDevice, st));
+        const size_t at = off + (size_t)i * item, bytes = (size_t)std::min(slice, cnt - i) * item;
+        memcpy(stage + at, chunk + at, bytes);
+        EKZG_CUDA(cudaMemcpyAsync(dev + at, stage + at, bytes, cudaMemcpyHostToDevice, st));
     }
     return Status::Ok();
 }
+
+static Status upload_blobs(Workspace& ws, const uint8_t* chunk, int o, int cnt, bool src_pinned, cudaStream_t st) {
+    return upload(ws.d_blobs, ws.h_blobs, chunk, BYTES_PER_BLOB, o, cnt, src_pinned, st);
+}
+
+// Blobs of the first FK20 piece of a chunk of cnt: its K1, K2 and K4 run while the rest of the chunk is still on the wire.  A
+// quarter of the chunk (whole 32-blob groups) from 512 blobs up, else the whole chunk.
+static int fk20_first_piece(int cnt) { return cnt >= 512 ? ((cnt / 4 + 31) & ~31) : cnt; }
 
 // The batch scheduler behind every host-buffer prover entry point (replaces the reference's rayon fan-out,
 // crates/maybe_rayon/src/multi_threaded.rs:9-39).  A chunk (<= EKZG_CHUNK blobs, default 1024) is cut into
@@ -631,7 +678,7 @@ Status Context::compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* bl
         int* off = piece_off[slot];
         int* len = piece_len[slot];
         if (want_proofs) {
-            const int q = cnt >= 512 ? ((cnt / 4 + 31) & ~31) : cnt;
+            const int q = fk20_first_piece(cnt);
             off[np] = 0; len[np++] = q;
             if (q < cnt) { off[np] = q; len[np++] = cnt - q; }
         } else {   // cells only: nothing but copies and K1, finer pieces keep both copy engines busy
@@ -1078,7 +1125,7 @@ Status Context::run_4844(Mode4844 mode, uint64_t n, const uint8_t* blobs, const 
         if (mode != Mode4844::BlobProof) EKZG_CUDA(cudaMemsetAsync(ws.d_status2, 0, sizeof(uint32_t) * cnt, st));
         EKZG_CUDA(launch_blob_to_coeffs_cells(ws.d_blobs, ws.d_coeffs, nullptr, ws.d_status, T_, cnt, false, st));
         if (mode == Mode4844::Commit) {
-            EKZG_CUDA(launch_coeffs_to_scalars(ws.d_coeffs, ws.d_scalars, cnt, st));
+            EKZG_TRY(commit_device(ws, cnt, ws.d_out48, st));
         } else {
             if (mode == Mode4844::BlobProof && n <= (uint64_t)HOST_CHALLENGE_MAX) {
                 // a handful of blobs: Fiat-Shamir challenges on the host (see host_blob_challenge), uploaded like user-supplied points
@@ -1094,10 +1141,8 @@ Status Context::run_4844(Mode4844 mode, uint64_t n, const uint8_t* blobs, const 
                 EKZG_CUDA(launch_scalars_from_be(ws.d_z32, ws.d_z, ws.d_status2, cnt, st));
             }
             EKZG_CUDA(launch_quotient(ws.d_coeffs, ws.d_z, ws.d_scalars, mode == Mode4844::PointProof ? ws.d_z32 : nullptr, cnt, st));
+            EKZG_TRY(srs_msm_compress(ws, cnt, ws.d_out48, st));
         }
-        EKZG_CUDA(launch_fixed_msm(ws.d_scalars, ws.d_pts, T_.srs, N_BLOB / FK20_POINTS, cnt, st, 0, -1, ws.d_msm_scratch));
-        EKZG_CUDA(launch_sum_positions(ws.d_pts, cnt, N_BLOB / FK20_POINTS, 2, st));
-        EKZG_CUDA(launch_g1_compress(ws.d_pts, ws.d_out48, 1, cnt, st));
         EKZG_CUDA(cudaMemcpyAsync(out48 + first * 48, ws.d_out48, (size_t)cnt * 48, cudaMemcpyDeviceToHost, st));
         if (mode == Mode4844::PointProof) EKZG_CUDA(cudaMemcpyAsync(out_y32 + first * 32, ws.d_z32, (size_t)cnt * 32, cudaMemcpyDeviceToHost, st));
         if (mode == Mode4844::BlobProof) EKZG_CUDA(cudaStreamWaitEvent(st, ws.sub_out[0], 0));
@@ -1131,6 +1176,166 @@ Status Context::compute_blob_kzg_proof_batch(uint64_t n, const uint8_t* blobs, c
 Status Context::compute_kzg_proof_batch(uint64_t n, const uint8_t* blobs, const uint8_t* z32, uint8_t* out_proof48, uint8_t* out_y32,
                                         uint8_t* item_status) const {
     return run_4844(Mode4844::PointProof, n, blobs, z32, out_proof48, out_y32, item_status);
+}
+
+// ------------------------------------------------------------------------------------------------
+// The cell proofs of whole blobs, by recomputation: a blob has exactly one valid proof per cell, and the FK20 pipeline computes
+// all 128 of them, so the check is a byte comparison -- no cells cross PCIe, no transcript hash, no randomness, and a verdict per
+// cell.  Chunks and the two alternating workspaces as in compute_cells_and_kzg_proofs_batch; all kernels of a chunk on ws.stream.
+Status Context::verify_blob_cell_proofs_batch(uint64_t n, const uint8_t* blobs, const uint8_t* commitments, const uint8_t* proofs,
+                                              uint8_t* item_status, uint8_t* cell_status, bool* all_ok) const {
+    *all_ok = n == 0;
+    if (n == 0) return Status::Ok();
+    EKZG_TRY(bind_device());
+    const int cap = (int)std::min<uint64_t>(n, (uint64_t)chunk_capacity());
+    const uint64_t nchunks = (n + cap - 1) / cap;
+    const ProofRoute route = proof_route(n, cap, true);
+    Workspace* W[2] = {acquire(route.capacity, true), nchunks > 1 ? acquire(cap, true) : nullptr};
+    Status result = Status::Ok();
+    if (!W[0] || (nchunks > 1 && !W[1])) result = Status::Error("device/pinned memory allocation failed");
+    for (Workspace* w : W)
+        if (w && result.ok) result = w->ensure_verify_buffers(cap);
+    if (!result.ok) {
+        for (Workspace* w : W) if (w) give_back(w, result);
+        return result;
+    }
+    const bool blobs_pinned = host_range_is_pinned(blobs), c_pinned = host_range_is_pinned(commitments), p_pinned = host_range_is_pinned(proofs);
+    std::vector<uint8_t> cell_mm((size_t)n * N_CELLS), blob_mm(n);
+    TraceClock tr("verify_blob_cell_proofs_batch");
+    uint64_t pending_first[2] = {0, 0};
+    int pending_cnt[2] = {0, 0};
+    auto drain = [&](int slot) -> Status {
+        Workspace& ws = *W[slot];
+        if (!pending_cnt[slot]) return Status::Ok();
+        EKZG_CUDA(cudaEventSynchronize(ws.done));
+        memcpy(&cell_mm[pending_first[slot] * N_CELLS], ws.h_cell_mm, (size_t)pending_cnt[slot] * N_CELLS);
+        memcpy(&blob_mm[pending_first[slot]], ws.h_blob_mm, (size_t)pending_cnt[slot]);
+        pending_cnt[slot] = 0;
+        return Status::Ok();
+    };
+    auto submit = [&](int slot, uint64_t first, int cnt) -> Status {
+        Workspace& ws = *W[slot];
+        const cudaStream_t st = ws.stream;
+        EKZG_CUDA(cudaStreamWaitEvent(ws.in_stream, ws.done, 0));
+        EKZG_CUDA(cudaMemsetAsync(ws.d_status, 0, sizeof(uint32_t) * cnt, st));
+        // the blobs in the prover's pieces: K1 (once: the coefficients both the proofs and the commitment are computed from), K2
+        // and K4 of the first piece run while the rest is on the wire
+        const int q = fk20_first_piece(cnt);
+        const int off[2] = {0, q}, len[2] = {q, cnt - q};
+        for (int s = 0; s < 2 && len[s]; s++) {
+            EKZG_TRY(upload(ws.d_blobs, ws.h_blobs, blobs + first * BYTES_PER_BLOB, BYTES_PER_BLOB, off[s], len[s], blobs_pinned, ws.in_stream));
+            EKZG_CUDA(cudaEventRecord(ws.piece_in[s], ws.in_stream));
+            EKZG_CUDA(cudaStreamWaitEvent(st, ws.piece_in[s], 0));
+            EKZG_CUDA(launch_blob_to_coeffs_cells(ws.d_blobs + (size_t)off[s] * BYTES_PER_BLOB, ws.d_coeffs + (size_t)off[s] * N_BLOB, nullptr,
+                                                  ws.d_status + off[s], T_, len[s], false, st));
+            if (!route.direct) EKZG_TRY(fk20_msm(ws, cnt, off[s], len[s], st, nullptr));
+        }
+        EKZG_TRY(upload(ws.d_given_proofs, ws.h_proofs, proofs + first * PROOFS_PER_BLOB, PROOFS_PER_BLOB, 0, cnt, p_pinned, ws.in_stream));
+        EKZG_TRY(upload(ws.d_c48, ws.h_c48, commitments + first * BYTES_PER_G1, BYTES_PER_G1, 0, cnt, c_pinned, ws.in_stream));
+        EKZG_CUDA(cudaEventRecord(ws.piece_in[2], ws.in_stream));   // (after the two pieces of blobs)
+        if (route.direct) EKZG_TRY(proofs_direct_device(ws, cnt, ws.d_proofs, st));
+        else EKZG_TRY(fk20_ntt_compress(ws, cnt, ws.d_proofs, st, nullptr));
+        // The commitment reuses d_scalars and d_pts, which the proofs are done with once they are compressed (K6, or the direct
+        // route's compression).  d_coeffs is still intact: K2 and the direct route's quotient kernel only read it.  On the direct
+        // route the workspace holds 128 cnt "virtual blobs", far more than the cnt items of the commitment MSM.
+        EKZG_TRY(commit_device(ws, cnt, ws.d_out48, st));
+        EKZG_CUDA(cudaStreamWaitEvent(st, ws.piece_in[2], 0));   // the supplied proofs and commitments are on the device
+        EKZG_CUDA(launch_compare_blob_proofs(ws.d_proofs, ws.d_given_proofs, ws.d_out48, ws.d_c48, ws.d_status, ws.d_cell_mm, ws.d_blob_mm, cnt, st));
+        EKZG_CUDA(cudaMemcpyAsync(ws.h_cell_mm, ws.d_cell_mm, (size_t)cnt * N_CELLS, cudaMemcpyDeviceToHost, st));
+        EKZG_CUDA(cudaMemcpyAsync(ws.h_blob_mm, ws.d_blob_mm, (size_t)cnt, cudaMemcpyDeviceToHost, st));
+        EKZG_CUDA(cudaEventRecord(ws.done, st));
+        pending_first[slot] = first;
+        pending_cnt[slot] = cnt;
+        return Status::Ok();
+    };
+    for (uint64_t c = 0; c < nchunks && result.ok; c++) {
+        const int slot = (int)(c & 1);
+        result = drain(slot);
+        if (result.ok) result = submit(slot, c * cap, (int)std::min<uint64_t>(cap, n - c * cap));
+    }
+    for (int slot = 0; slot < 2 && result.ok; slot++)
+        if (W[slot]) result = drain(slot);
+    tr.mark("H2D + kernels + D2H of the chunks");
+
+    // Phase B, only where a comparison failed: is the differing encoding a valid point (verdict 1) or not (2)?  A byte-equal
+    // encoding needs no check -- the library's own compression output is canonical and valid -- so an honest batch launches no
+    // validation kernel.  Encodings of non-canonical blobs are skipped: those items are 2 whatever they hold.
+    std::vector<uint8_t> enc;
+    for (uint64_t i = 0; i < n && result.ok; i++) {
+        if (blob_mm[i] & BLOB_MM_NON_CANONICAL) continue;
+        if (blob_mm[i] & BLOB_MM_COMMITMENT) enc.insert(enc.end(), commitments + i * BYTES_PER_G1, commitments + (i + 1) * BYTES_PER_G1);
+        if (blob_mm[i] & BLOB_MM_PROOF)
+            for (int k = 0; k < N_CELLS; k++)
+                if (cell_mm[i * N_CELLS + k]) {
+                    const uint8_t* p = proofs + (i * N_CELLS + k) * BYTES_PER_G1;
+                    enc.insert(enc.end(), p, p + BYTES_PER_G1);
+                }
+    }
+    const size_t m = enc.size() / BYTES_PER_G1;
+    tr.mark("phase B: gather");
+    std::vector<uint32_t> invalid(m);
+    if (m && result.ok) {
+        uint8_t* d_enc = nullptr;
+        G1Affine* d_aff = nullptr;
+        uint32_t* d_st = nullptr;
+        const cudaStream_t st = W[0]->stream;
+        // stream-ordered allocations: cudaMalloc / cudaFree would wait for the work of every other caller on the device
+        auto validate = [&]() -> Status {
+            EKZG_CUDA(cudaMallocAsync(&d_enc, enc.size(), st));
+            EKZG_CUDA(cudaMallocAsync(&d_aff, m * sizeof(G1Affine), st));
+            EKZG_CUDA(cudaMallocAsync(&d_st, m * sizeof(uint32_t), st));
+            EKZG_CUDA(cudaMemcpyAsync(d_enc, enc.data(), enc.size(), cudaMemcpyHostToDevice, st));
+            EKZG_CUDA(launch_g1_validate(d_enc, d_aff, d_st, (int)m, true, st));
+            EKZG_CUDA(cudaMemcpyAsync(invalid.data(), d_st, m * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+            return Status::Ok();
+        };
+        result = validate();
+        for (void* p : {(void*)d_enc, (void*)d_aff, (void*)d_st}) if (p) cudaFreeAsync(p, st);
+        const cudaError_t e = cudaStreamSynchronize(st);   // (also when a step failed: the copies may still read `enc` / write `invalid`)
+        if (result.ok && e != cudaSuccess) result = Status::Error(std::string("CUDA error: ") + cudaGetErrorString(e) + " in phase B");
+        if (!result.ok) cudaGetLastError();
+        tr.mark("phase B: validate");
+    }
+    for (Workspace* w : W) if (w) give_back(w, result);
+    if (!result.ok) return result;
+
+    // The verdicts.  Why comparing bytes decides what the reference verifier decides, opening by opening:
+    //  - C = commit(p): the single-cell equation e(C - [I_k(tau)]_1, [1]_2) = e(pi, [tau^64 - h_k^64]_2) has exactly one solution
+    //    pi (the G2 factor is not the identity, and pairing with it is injective on G1), and that solution is [q_k(tau)], the FK20
+    //    output for cell k.  So cell verdict 0 <=> the reference accepts that opening, exactly.
+    //  - C != commit(p): the reference could accept all 128 openings only if C opened to p at all 8192 points, i.e. C committed to
+    //    p -- a break of KZG binding.  So the blob verdicts agree except on inputs nobody can produce.
+    //  - Where the two differ: per opening, with C != commit(p), the reference can accept opening k (for example when C commits to
+    //    p + c (X^64 - h_k^64), which agrees with p on coset k); this call reports the blob as failing and the cell by its proof.
+    //  - The reference's batch check is itself probabilistic (error <= n / |Fr|); this one is deterministic.
+    // cell_status therefore states a fact about the proof and the blob alone and does not depend on C.
+    bool ok = true;
+    size_t j = 0;   // walks `invalid` in the order phase B gathered the encodings
+    for (uint64_t i = 0; i < n; i++) {
+        uint8_t* cs = &cell_mm[i * N_CELLS];
+        uint8_t v = VERDICT_OK;
+        if (blob_mm[i] & BLOB_MM_NON_CANONICAL) {
+            v = VERDICT_MALFORMED;   // (the kernel wrote 2 for every cell)
+        } else {
+            bool malformed = false, fails = false;
+            if (blob_mm[i] & BLOB_MM_COMMITMENT) (invalid[j++] ? malformed : fails) = true;
+            if (blob_mm[i] & BLOB_MM_PROOF)
+                for (int k = 0; k < N_CELLS; k++)
+                    if (cs[k]) {
+                        cs[k] = invalid[j++] ? VERDICT_MALFORMED : VERDICT_FAILS;
+                        (cs[k] == VERDICT_MALFORMED ? malformed : fails) = true;
+                    }
+            v = malformed ? VERDICT_MALFORMED : (fails ? VERDICT_FAILS : VERDICT_OK);
+        }
+        item_status[i] = v;
+        ok = ok && v == VERDICT_OK;
+    }
+    // the gather loop and this one must visit the mismatches in the same order: if they ever disagree, fail rather than hand
+    // out verdicts that belong to other encodings
+    if (j != m) return Status::Error("verify_blob_cell_proofs_batch: phase B consumed " + std::to_string(j) + " of " + std::to_string(m) + " validations");
+    if (cell_status) memcpy(cell_status, cell_mm.data(), cell_mm.size());
+    *all_ok = ok;
+    return Status::Ok();
 }
 
 }  // namespace ekzg

@@ -100,6 +100,18 @@ struct Workspace {
     bool recover_ready = false;    // all six recovery buffers exist
     Status ensure_recover_buffers();
     void free_recover_buffers();
+    // verify_blob_cell_proofs_batch (allocated on first use, for the blobs per chunk a call needs -- not the workspace capacity,
+    // which on the direct route counts 128 "virtual blobs" per blob; the supplied commitments go to d_c48, pageable proofs are
+    // staged in h_proofs)
+    uint8_t* d_given_proofs = nullptr;   // [vcap][128][48]
+    uint8_t* d_cell_mm = nullptr;        // [vcap][128] per-cell comparison bytes, then d_blob_mm
+    uint8_t* d_blob_mm = nullptr;        // [vcap] per-blob BLOB_MM_* bits
+    uint8_t* h_cell_mm = nullptr;        // pinned, the same layout
+    uint8_t* h_blob_mm = nullptr;
+    uint8_t* h_c48 = nullptr;            // pinned staging of pageable commitments
+    int verify_capacity = 0;             // vcap: blobs the buffers hold (0: none allocated)
+    Status ensure_verify_buffers(int blobs);   // (re)allocates when fewer than `blobs` (<= capacity) fit
+    void free_verify_buffers();
     // pinned host staging (the ABI hands us scattered caller buffers)
     uint8_t* h_blobs = nullptr;
     uint8_t* h_cells = nullptr;
@@ -178,6 +190,12 @@ public:
     // item_status (mode 1 only, optional): a Verdict per item instead of Err for malformed items; *verified = all are VERDICT_OK.
     Status verify_kzg_proofs(int mode, uint64_t n, const uint8_t* const* blobs, const uint8_t* const* commitments, const uint8_t* z32,
                              const uint8_t* y32, const uint8_t* const* proofs, bool* verified, uint8_t* item_status = nullptr) const;
+    // The cell proofs of whole blobs (an EIP-7594 blob transaction): recomputes each blob's commitment and 128 proofs and compares
+    // bytes.  Host buffers, contiguous: blobs n x 131072 B, commitments n x 48 B, proofs n x 128 x 48 B.  item_status[n]: a Verdict
+    // per blob; cell_status[n][128] (optional): 0 the proof of cell k, 1 a valid point but not that proof, 2 not a valid encoding or
+    // a non-canonical blob.  *all_ok = every item is VERDICT_OK.  Err only for allocation / CUDA failures.
+    Status verify_blob_cell_proofs_batch(uint64_t n, const uint8_t* blobs, const uint8_t* commitments, const uint8_t* proofs,
+                                         uint8_t* item_status, uint8_t* cell_status, bool* all_ok) const;
 
     // workspace pool (calls are re-entrant: concurrent callers each borrow their own workspaces)
     Workspace* acquire(int min_capacity, bool with_io) const;
@@ -215,6 +233,10 @@ private:
     Status fk20_from_coeffs_device(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream,
                                    std::vector<cudaEvent_t>* stage_events = nullptr) const;
     Status proofs_direct_device(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream) const;   // needs ws.capacity >= 128 n
+    // commitments of n blobs from ws.d_coeffs into d_out48 (n x 48 B), asynchronous on `stream`; uses ws.d_scalars and ws.d_pts
+    Status commit_device(Workspace& ws, int n, uint8_t* d_out48, cudaStream_t stream) const;
+    // B 4096-point MSMs over the SRS tables from the scalars in ws.d_scalars ([4096][B] plain), compressed into d_out (B x 48 B)
+    Status srs_msm_compress(Workspace& ws, int B, uint8_t* d_out, cudaStream_t stream) const;
     // K2 + K4 of blobs [o, o + c) of an n-blob batch (c < 0: to the end), then K5 + K6 of all n; stage events 2..5 as in fk20_device
     Status fk20_msm(Workspace& ws, int n, int o, int c, cudaStream_t stream, std::vector<cudaEvent_t>* stage_events) const;
     Status fk20_ntt_compress(Workspace& ws, int n, uint8_t* d_proofs, cudaStream_t stream, std::vector<cudaEvent_t>* stage_events) const;

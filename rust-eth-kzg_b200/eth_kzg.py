@@ -69,7 +69,8 @@ def load_library():
                  "eth_kzg_b200_recover_cells_and_kzg_proofs_batch", "eth_kzg_b200_blob_to_kzg_commitment_batch", "eth_kzg_b200_compute_blob_kzg_proof_batch",
                  "eth_kzg_b200_das_context_new_from_json", "eth_kzg_b200_debug_parse_trusted_setup_json", "eth_kzg_b200_debug_g2_keys"):
         getattr(lib, name).restype = _CResult
-    for name in ("eth_kzg_b200_verify_cell_kzg_proof_batch_groups", "eth_kzg_b200_verify_blob_kzg_proof_batch_items"):
+    for name in ("eth_kzg_b200_verify_cell_kzg_proof_batch_groups", "eth_kzg_b200_verify_blob_kzg_proof_batch_items",
+                 "eth_kzg_b200_verify_blob_cell_proofs_batch"):
         if hasattr(lib, name):   # (an EKZG_LIB build from before these entry points lacks them)
             getattr(lib, name).restype = _CResult
     _lib = lib
@@ -306,6 +307,22 @@ class DASContext:
                                                                                    C.byref(ok)))
         del k1, k2, k3
         return bool(ok.value), list(status.raw[:n])
+
+    def verify_blob_cell_proofs_batch(self, blobs_flat, commitments_flat, proofs_flat, n, want_cells=False):
+        """the 128 cell proofs of each of n blobs (an EIP-7594 blob transaction), checked by recomputing them on the device.
+        Contiguous bytes: n*131072 B of blobs, n*48 B of commitments, n*128*48 B of proofs in cell order.
+        -> (all_ok, [status per blob], cell status bytes (n*128) or None): a blob is 0 verifies, 1 does not, 2 malformed
+        (non-canonical blob, invalid commitment or proof); a cell is 0 its proof, 1 a valid point but not its proof, 2 an invalid
+        encoding or a non-canonical blob.  Raises KzgError only on infrastructure errors."""
+        blobs_flat = _exact(blobs_flat, n * BYTES_PER_BLOB, "blobs")
+        commitments_flat = _exact(commitments_flat, n * 48, "commitments")
+        proofs_flat = _exact(proofs_flat, n * CELLS_PER_EXT_BLOB * 48, "proofs")
+        status = C.create_string_buffer(max(n, 1))
+        cells = C.create_string_buffer(max(n, 1) * CELLS_PER_EXT_BLOB) if want_cells else None
+        ok = C.c_bool(False)
+        _check(self._lib, self._lib.eth_kzg_b200_verify_blob_cell_proofs_batch(C.c_void_p(self._ctx), C.c_uint64(n), blobs_flat, commitments_flat,
+                                                                               proofs_flat, status, cells, C.byref(ok)))
+        return bool(ok.value), list(status.raw[:n]), (cells.raw[:n * CELLS_PER_EXT_BLOB] if want_cells else None)
 
     # ---- additive batch / device entry points --------------------------------------------------
     def compute_cells_and_kzg_proofs_batch(self, blobs_flat, n, want_proofs=True):

@@ -8,7 +8,8 @@ kernels when their files are equal.
 Calls: compute_cells_and_kzg_proofs batch (1, 2, 8, 33, 1024 blobs), the device entry point (1, 1024), recovery batch
 (1, 40), blob_to_kzg_commitment batch and compute_blob_kzg_proof batch (1, 40), compute_kzg_proof (1 call, 40 calls), the
 verifiers verify_cell_kzg_proof_batch (128 and 16 384 openings) and verify_blob_kzg_proof_batch (1, 20 blobs), and, where the
-build has them, the grouped cell verifier and the per-blob verifier on the same inputs (honest, and with one bad item).
+build has them, the grouped cell verifier and the per-blob verifier on the same inputs (honest, and with one bad item), and
+verify_blob_cell_proofs_batch on 20 blobs (honest, and with one bad proof).
 Each call runs once before it is counted, so first-use allocations are not part of it."""
 import argparse
 import ctypes as C
@@ -119,6 +120,12 @@ def main():
         swapped = bpl[:1] + [bpl[2], bpl[1]] + bpl[3:]
         for name, pl in (("honest", bpl), ("one_bad", swapped)):
             res["verify_blobs_items_20_%s" % name] = record(lib, lambda pl=pl: ctx.verify_blob_kzg_proof_batch_items(bl, bcl, pl))
+    if hasattr(lib, "eth_kzg_b200_verify_blob_cell_proofs_batch"):
+        cp = proofs[:20 * 128 * 48]
+        cp_bad = cp[:48] + cp[2 * 48:3 * 48] + cp[2 * 48:]   # blob 0: the proof of cell 2 in place of cell 1
+        for name, p in (("honest", cp), ("one_bad", cp_bad)):
+            res["verify_blob_cell_proofs_20_%s" % name] = record(
+                lib, lambda p=p: ctx.verify_blob_cell_proofs_batch(flat[:20 * 131072], cms[:20 * 48], p, 20, want_cells=True))
     ctx.close()
 
     with open(args.out, "w") as f:
