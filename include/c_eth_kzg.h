@@ -154,6 +154,20 @@ CResult eth_kzg_b200_recover_cells_and_kzg_proofs_batch(const DASContext *ctx, u
                                                         const uint64_t *cell_indices, const uint8_t *cells, uint8_t *out_cells,
                                                         uint8_t *out_proofs, uint8_t *item_status);
 
+/* Blobs from their cells without computing cell proofs: what a node that holds at least 64 of the 128 data columns needs to
+ * serve blobs (cell_0 || ... || cell_63 == blob).  Inputs, validation order, item_status values and error messages are those
+ * of eth_kzg_b200_recover_cells_and_kzg_proofs_batch: cell_counts[n], cell_indices and cells (2048 B each) of all blobs
+ * concatenated in blob order.  out_blobs: n*131072 B, contiguous; for every valid item, cells 0..63 of what the proofs call
+ * returns; the blobs of invalid items are unspecified.  item_status[n] (optional): 0 ok, 3 invalid indices, 1 non-canonical
+ * cell scalar, 4 recovered polynomial of degree >= 4096.  Err iff any item is invalid (the message the proofs call returns for
+ * the same inputs).  n = 0 gives Ok.  Pinned caller buffers are DMA'd as they are; pageable ones are staged. */
+CResult eth_kzg_b200_recover_blobs_batch(const DASContext *ctx, uint64_t n, const uint64_t *cell_counts, const uint64_t *cell_indices,
+                                         const uint8_t *cells, uint8_t *out_blobs, uint8_t *item_status);
+/* One blob from its cells, shaped like eth_kzg_recover_cells_and_proofs (an array of cell pointers) with the same checks
+ * (length mismatch, more than 4096 cells) and errors.  out_blob: 131072 B. */
+CResult eth_kzg_b200_recover_blob(const DASContext *ctx, uint64_t cells_length, const uint8_t *const *cells, uint64_t cell_indices_length,
+                                  const uint64_t *cell_indices, uint8_t *out_blob);
+
 /* verify_cell_kzg_proof_batch with a verdict per caller-defined group of openings (for example the cells of one column
  * sidecar).  Inputs as eth_kzg_verify_cell_kzg_proof_batch (n of each), plus group_of[n] (< n_groups).  group_status[n_groups]:
  * 0 every opening of the group verifies (also: an empty group), 1 the group's openings do not verify, 2 the group holds a

@@ -295,6 +295,21 @@ CResult eth_kzg_b200_recover_cells_and_kzg_proofs_batch(const DASContext* ctx, u
     DeviceGuard guard;
     return to_c(ds(ctx).recover_cells_and_kzg_proofs_batch(n, cell_counts, cell_indices, cells, out_cells, out_proofs, item_status));
 }
+CResult eth_kzg_b200_recover_blobs_batch(const DASContext* ctx, uint64_t n, const uint64_t* cell_counts, const uint64_t* cell_indices,
+                                         const uint8_t* cells, uint8_t* out_blobs, uint8_t* item_status) {
+    DeviceGuard guard;
+    return to_c(ds(ctx).recover_blobs_batch(n, cell_counts, cell_indices, cells, out_blobs, item_status));
+}
+CResult eth_kzg_b200_recover_blob(const DASContext* ctx, uint64_t cells_length, const uint8_t* const* cells, uint64_t cell_indices_length,
+                                  const uint64_t* cell_indices, uint8_t* out_blob) {
+    DeviceGuard guard;
+    const ekzg::Context& c = next_cx(ctx);
+    if (cells_length != cell_indices_length) return c_err("Recovery(NumCellIndicesNotEqualToNumCells)");   // as eth_kzg_recover_cells_and_proofs
+    if (cells_length > 4096) return c_err("Recovery(TooManyCellsReceived)");
+    std::vector<uint8_t> flat((size_t)cells_length * ekzg::BYTES_PER_CELL);
+    for (uint64_t i = 0; i < cells_length; i++) memcpy(flat.data() + i * ekzg::BYTES_PER_CELL, cells[i], ekzg::BYTES_PER_CELL);
+    return to_c(c.recover_blobs_batch(1, &cells_length, cell_indices, flat.data(), out_blob, nullptr));
+}
 
 CResult eth_kzg_verify_cell_kzg_proof_batch(const DASContext* ctx, uint64_t commitments_length, const uint8_t* const* commitments,
                                             uint64_t cell_indices_length, const uint64_t* cell_indices, uint64_t cells_length,

@@ -93,6 +93,27 @@ k_blob_to_coeffs_cells(const uint8_t* __restrict__ blobs, Fr* __restrict__ coeff
     }
 }
 
+// Half `halfsel` of the 8192-point extension of one blob's coefficients cf, as big-endian bytes at out: BRP(NTT_4096(c))
+// (halfsel 0: cells 0..63, i.e. the blob) or BRP(NTT_4096(c[i] w8192^i)) (halfsel 1: cells 64..127).  sm: 128 KiB.
+__device__ __forceinline__ void coeffs_half_to_be(const Fr* __restrict__ cf, uint8_t* __restrict__ out, int halfsel, const DevTables& T,
+                                                  uint32_t* sm, int tid) {
+    for (int i = tid; i < N_BLOB; i += K1_THREADS) {
+        Fr c = ld_vec(&cf[i]);
+        if (halfsel) {
+            Fr w = ld_vec(&T.tw8192[i]);
+            fe_mul(c, c, w);
+        }
+        smem_st(sm, N_BLOB, i, c);
+    }
+    __syncthreads();
+    ntt_dif_shared<12>(sm, N_BLOB, 1, T.tw4096, tid, K1_THREADS);
+    for (int i = tid; i < N_BLOB; i += K1_THREADS) {
+        Fr v = smem_ld(sm, N_BLOB, i);
+        fe_from_mont(v, v);
+        fr_store_be(out + (size_t)i * 32, v);
+    }
+}
+
 // coefficients -> all 128 cells (recovery path: Input::PolyCoeff, fk20/prover.rs:184-188 + 158-165)
 __global__ void __launch_bounds__(K1_THREADS, 1)
 k_coeffs_to_cells(const Fr* __restrict__ coeffs, uint8_t* __restrict__ cells, DevTables T) {
@@ -101,23 +122,17 @@ k_coeffs_to_cells(const Fr* __restrict__ coeffs, uint8_t* __restrict__ cells, De
     const Fr* cf = coeffs + (size_t)b * N_BLOB;
     uint8_t* out = cells + (size_t)b * (N_EXT * 32);
     for (int halfsel = 0; halfsel < 2; halfsel++) {
-        for (int i = tid; i < N_BLOB; i += K1_THREADS) {
-            Fr c = ld_vec(&cf[i]);
-            if (halfsel) {
-                Fr w = ld_vec(&T.tw8192[i]);
-                fe_mul(c, c, w);
-            }
-            smem_st(sm, N_BLOB, i, c);
-        }
-        __syncthreads();
-        ntt_dif_shared<12>(sm, N_BLOB, 1, T.tw4096, tid, K1_THREADS);
-        for (int i = tid; i < N_BLOB; i += K1_THREADS) {
-            Fr v = smem_ld(sm, N_BLOB, i);
-            fe_from_mont(v, v);
-            fr_store_be(out + (size_t)(halfsel * N_BLOB + i) * 32, v);
-        }
+        coeffs_half_to_be(cf, out + (size_t)halfsel * BYTES_PER_BLOB, halfsel, T, sm, tid);
         __syncthreads();
     }
+}
+
+// coefficients -> the blob (cells 0..63 only: half the transforms and half the bytes of k_coeffs_to_cells)
+__global__ void __launch_bounds__(K1_THREADS, 1)
+k_coeffs_to_blob(const Fr* __restrict__ coeffs, uint8_t* __restrict__ blobs, DevTables T) {
+    extern __shared__ uint32_t sm[];
+    const int b = blockIdx.x;
+    coeffs_half_to_be(coeffs + (size_t)b * N_BLOB, blobs + (size_t)b * BYTES_PER_BLOB, 0, T, sm, threadIdx.x);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1413,7 +1428,9 @@ cudaError_t kernels_init() {
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(k_fk20_g1_ntts_vm, cudaFuncAttributeMaxDynamicSharedMemorySize, fpvm::SMEM_BYTES);
     if (e != cudaSuccess) return e;
-    return cudaFuncSetAttribute(k_coeffs_to_cells, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * N_BLOB * 4);
+    e = cudaFuncSetAttribute(k_coeffs_to_cells, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * N_BLOB * 4);
+    if (e != cudaSuccess) return e;
+    return cudaFuncSetAttribute(k_coeffs_to_blob, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * N_BLOB * 4);
 }
 
 cudaError_t launch_blob_to_coeffs_cells(const uint8_t* blobs, Fr* coeffs, uint8_t* cells, uint32_t* status, const DevTables& T,
@@ -1425,6 +1442,12 @@ cudaError_t launch_blob_to_coeffs_cells(const uint8_t* blobs, Fr* coeffs, uint8_
 
 cudaError_t launch_coeffs_to_cells(const Fr* coeffs, uint8_t* cells, const DevTables& T, int B, cudaStream_t st) {
     k_coeffs_to_cells<<<B, K1_THREADS, 8 * N_BLOB * 4, st>>>(coeffs, cells, T);
+    EKZG_LAUNCH_CHECK();
+    return cudaSuccess;
+}
+
+cudaError_t launch_coeffs_to_blob(const Fr* coeffs, uint8_t* blobs, const DevTables& T, int B, cudaStream_t st) {
+    k_coeffs_to_blob<<<B, K1_THREADS, 8 * N_BLOB * 4, st>>>(coeffs, blobs, T);
     EKZG_LAUNCH_CHECK();
     return cudaSuccess;
 }

@@ -19,6 +19,7 @@ cudaError_t launch_powers(Fr* out, const uint32_t* base_mont, int n, cudaStream_
 cudaError_t launch_blob_to_coeffs_cells(const uint8_t* blobs, Fr* coeffs, uint8_t* cells, uint32_t* status, const DevTables& T,
                                         int B, bool want_cells, cudaStream_t st);
 cudaError_t launch_coeffs_to_cells(const Fr* coeffs, uint8_t* cells, const DevTables& T, int B, cudaStream_t st);
+cudaError_t launch_coeffs_to_blob(const Fr* coeffs, uint8_t* blobs, const DevTables& T, int B, cudaStream_t st);   // cells 0..63 only
 // blobs [b0, b0 + cnt) of a batch of B (cnt < 0: to the end)
 cudaError_t launch_toeplitz_scalars(const Fr* coeffs, uint32_t* scalars, const DevTables& T, int B, cudaStream_t st, int b0 = 0, int cnt = -1);
 // scratch: fixed_msm_scratch_bytes(T) bytes for the batched-affine kernel (nullptr: the XYZZ kernels are used)
@@ -50,7 +51,7 @@ cudaError_t launch_g1_validate(const uint8_t* in, G1Affine* out, uint32_t* statu
 cudaError_t recover_kernels_init();
 cudaError_t launch_recover_coeffs(const uint8_t* cells, const int16_t* slotmap, Fr* ze, Fr* czinv, Fr* bufA, Fr* bufB, Fr* coeffs,
                                   uint32_t* status, const DevTables& T, const Fr* shift_fwd, const Fr* shift_inv, const uint32_t* gen64_mont,
-                                  int B, cudaStream_t st);
+                                  int B, cudaStream_t st, const uint32_t* cell_off = nullptr);
 
 // kzg_kernels_verify.cu
 cudaError_t launch_powers_from_hash(const uint8_t* hash, Fr* rpow, int n, cudaStream_t st);

@@ -83,15 +83,18 @@ constexpr int RN_THREADS = 1024;
 //  MODE 2: x[i] = bufA[rev13(i)] * 7^i / 8192; forward transform; out = value * czinv[rev13(q) % 128] -> bufB (bit-reversed)
 //  MODE 3: x[p] = bufB[rev13(p)]; inverse transform; c'[idx] = value * 7^-idx / 8192 at idx = rev13(q):
 //          idx >= 4096 must be zero (status |= 4 otherwise), idx < 4096 -> coeffs[b][idx]
-template <int MODE>
-__global__ void __launch_bounds__(RN_THREADS, 1)
-k_recover_ntt(const uint8_t* __restrict__ cells, const int16_t* __restrict__ slotmap, const Fr* __restrict__ ze, const Fr* __restrict__ czinv,
-              const Fr* __restrict__ src, Fr* __restrict__ dst, Fr* __restrict__ coeffs, uint32_t* __restrict__ status,
-              const Fr* __restrict__ shift, DevTables T) {
+//  The cells of MODE 1 lie in 128-slot rows (blob b's cell of slot s at cells[b][s]) or, PACKED, as the caller concatenated
+//  them: blob b's cell of slot s at cells[cell_off[b] + s].
+template <int MODE, bool PACKED>
+__device__ __forceinline__ void
+recover_ntt(const uint8_t* __restrict__ cells, const uint32_t* __restrict__ cell_off, const int16_t* __restrict__ slotmap,
+            const Fr* __restrict__ ze, const Fr* __restrict__ czinv, const Fr* __restrict__ src, Fr* __restrict__ dst,
+            Fr* __restrict__ coeffs, uint32_t* __restrict__ status, const Fr* __restrict__ shift, const DevTables& T) {
     extern __shared__ uint32_t sm[];
     const int b = blockIdx.x, h = blockIdx.y, tid = threadIdx.x;
     const Fr r2 = fe_const_r2<FrParams>();
     const Fr* tw_first = (MODE == 2) ? T.tw8192 : T.tw8192_inv;
+    const uint8_t* row = (MODE == 1) ? cells + (PACKED ? (size_t)cell_off[b] : (size_t)b * N_CELLS) * BYTES_PER_CELL : nullptr;
     bool bad = false;
     for (int i = tid; i < N_BLOB; i += RN_THREADS) {
         Fr x[2];
@@ -104,7 +107,7 @@ k_recover_ntt(const uint8_t* __restrict__ cells, const int16_t* __restrict__ slo
                 if (slot < 0) {
                     fe_set_zero(x[u]);
                 } else {
-                    Fr e = fr_load_be(cells + ((size_t)(b * 128 + slot) * BYTES_PER_CELL) + 32 * rbits(a, 6));
+                    Fr e = fr_load_be(row + (size_t)slot * BYTES_PER_CELL + 32 * rbits(a, 6));
                     bad |= fe_plain_ge_mod(e);
                     fe_mul(e, e, r2);
                     Fr z = ld_vec(&ze[b * 128 + mpos]);
@@ -154,26 +157,44 @@ k_recover_ntt(const uint8_t* __restrict__ cells, const int16_t* __restrict__ slo
     }
 }
 
+template <int MODE>
+__global__ void __launch_bounds__(RN_THREADS, 1)
+k_recover_ntt(const uint8_t* __restrict__ cells, const int16_t* __restrict__ slotmap, const Fr* __restrict__ ze, const Fr* __restrict__ czinv,
+              const Fr* __restrict__ src, Fr* __restrict__ dst, Fr* __restrict__ coeffs, uint32_t* __restrict__ status,
+              const Fr* __restrict__ shift, DevTables T) {
+    recover_ntt<MODE, false>(cells, nullptr, slotmap, ze, czinv, src, dst, coeffs, status, shift, T);
+}
+
+// R1 on packed cells: one H2D copy brings a run of blobs' cells up as the caller laid them out, with no re-layout on the host
+__global__ void __launch_bounds__(RN_THREADS, 1)
+k_recover_ntt_packed(const uint8_t* __restrict__ cells, const uint32_t* __restrict__ cell_off, const int16_t* __restrict__ slotmap,
+                     const Fr* __restrict__ ze, Fr* __restrict__ dst, uint32_t* __restrict__ status, DevTables T) {
+    recover_ntt<1, true>(cells, cell_off, slotmap, ze, nullptr, nullptr, dst, nullptr, status, nullptr, T);
+}
+
 
 cudaError_t recover_kernels_init() {
     cudaError_t e;
     if ((e = cudaFuncSetAttribute(k_recover_ntt<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * N_BLOB * 4)) != cudaSuccess) return e;
     if ((e = cudaFuncSetAttribute(k_recover_ntt<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * N_BLOB * 4)) != cudaSuccess) return e;
-    return cudaFuncSetAttribute(k_recover_ntt<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * N_BLOB * 4);
+    if ((e = cudaFuncSetAttribute(k_recover_ntt<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * N_BLOB * 4)) != cudaSuccess) return e;
+    return cudaFuncSetAttribute(k_recover_ntt_packed, cudaFuncAttributeMaxDynamicSharedMemorySize, 8 * N_BLOB * 4);
 }
 
-// cells: [B][128 slots][2048] wire bytes (slot = rank of the cell in the caller's list), slotmap: [B][128] slot of domain
-// position m = rev7(cell index) or -1.  bufA/bufB: [B][8192] Fr scratch.  Result: coeffs [B][4096], status bits 1 (cell
-// scalar not canonical) / 4 (recovered polynomial has degree >= 4096).
+// cells: [B][128 slots][2048] wire bytes (slot = rank of the cell in the caller's list), or with cell_off (packed) blob b's
+// cells from cells + cell_off[b] * 2048 on; slotmap: [B][128] slot of domain position m = rev7(cell index) or -1.
+// bufA/bufB: [B][8192] Fr scratch.  Result: coeffs [B][4096], status bits 1 (cell scalar not canonical) / 4 (recovered
+// polynomial has degree >= 4096).
 cudaError_t launch_recover_coeffs(const uint8_t* cells, const int16_t* slotmap, Fr* ze, Fr* czinv, Fr* bufA, Fr* bufB, Fr* coeffs,
                                   uint32_t* status, const DevTables& T, const Fr* shift_fwd, const Fr* shift_inv, const uint32_t* gen64_mont,
-                                  int B, cudaStream_t st) {
+                                  int B, cudaStream_t st, const uint32_t* cell_off) {
     Fr g;
     for (int i = 0; i < 8; i++) g.v[i] = gen64_mont[i];
     k_recover_prep<<<B, 128, 0, st>>>(slotmap, ze, czinv, T, g);
     EKZG_LAUNCH_CHECK();
     const size_t smem = 8 * N_BLOB * 4;
-    k_recover_ntt<1><<<dim3(B, 2), RN_THREADS, smem, st>>>(cells, slotmap, ze, czinv, nullptr, bufA, nullptr, status, nullptr, T);
+    if (cell_off) k_recover_ntt_packed<<<dim3(B, 2), RN_THREADS, smem, st>>>(cells, cell_off, slotmap, ze, bufA, status, T);
+    else k_recover_ntt<1><<<dim3(B, 2), RN_THREADS, smem, st>>>(cells, slotmap, ze, czinv, nullptr, bufA, nullptr, status, nullptr, T);
     EKZG_LAUNCH_CHECK();
     k_recover_ntt<2><<<dim3(B, 2), RN_THREADS, smem, st>>>(nullptr, slotmap, ze, czinv, bufA, bufB, nullptr, status, shift_fwd, T);
     EKZG_LAUNCH_CHECK();

@@ -134,15 +134,28 @@ Status DeviceSet::compute_blob_kzg_proof_batch(uint64_t n, const uint8_t* blobs,
     });
 }
 
-Status DeviceSet::recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
-                                                     uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const {
-    if (ctx_.size() == 1 || n <= 8) return ctx_[0]->recover_cells_and_kzg_proofs_batch(n, counts, indices, cells, out_cells, out_proofs, item_status);
+Status DeviceSet::fan_out_cells(uint64_t n, const uint64_t* counts,
+                                const std::function<Status(const Context&, uint64_t, uint64_t, uint64_t)>& fn) const {
+    if (ctx_.size() == 1 || n <= 8) return fn(*ctx_[0], 0, n, 0);
     std::vector<uint64_t> offset(n + 1, 0);   // blob i's cells and indices start at offset[i] in the concatenated inputs
     for (uint64_t i = 0; i < n; i++) offset[i + 1] = offset[i] + counts[i];
-    return fan_out(n, [&](const Context& c, uint64_t lo, uint64_t cnt) {
-        return c.recover_cells_and_kzg_proofs_batch(cnt, counts + lo, indices + offset[lo], cells + offset[lo] * BYTES_PER_CELL,
+    return fan_out(n, [&](const Context& c, uint64_t lo, uint64_t cnt) { return fn(c, lo, cnt, offset[lo]); });
+}
+
+Status DeviceSet::recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
+                                                     uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const {
+    return fan_out_cells(n, counts, [&](const Context& c, uint64_t lo, uint64_t cnt, uint64_t cell0) {
+        return c.recover_cells_and_kzg_proofs_batch(cnt, counts + lo, indices + cell0, cells + cell0 * BYTES_PER_CELL,
                                                     out_cells + lo * CELLS_PER_BLOB, out_proofs + lo * PROOFS_PER_BLOB,
                                                     item_status ? item_status + lo : nullptr);
+    });
+}
+
+Status DeviceSet::recover_blobs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells, uint8_t* out_blobs,
+                                      uint8_t* item_status) const {
+    return fan_out_cells(n, counts, [&](const Context& c, uint64_t lo, uint64_t cnt, uint64_t cell0) {
+        return c.recover_blobs_batch(cnt, counts + lo, indices + cell0, cells + cell0 * BYTES_PER_CELL, out_blobs + lo * BYTES_PER_BLOB,
+                                     item_status ? item_status + lo : nullptr);
     });
 }
 

@@ -34,6 +34,9 @@ public:
     // Runs fn(context, first item, item count) once per non-empty shard, shard 0 on the calling thread and the others on
     // threads of their own; returns the first failure in shard order.
     Status fan_out(uint64_t n, const std::function<Status(const Context&, uint64_t, uint64_t)>& fn) const;
+    // fan_out over items whose cells and indices are concatenated (counts[i] of item i): fn also gets the offset of the shard's
+    // first cell
+    Status fan_out_cells(uint64_t n, const uint64_t* counts, const std::function<Status(const Context&, uint64_t, uint64_t, uint64_t)>& fn) const;
 
     Status compute_cells_and_kzg_proofs_batch(uint64_t n, const uint8_t* blobs, uint8_t* cells, uint8_t* proofs, uint8_t* blob_status,
                                               bool want_proofs) const;
@@ -42,6 +45,8 @@ public:
                                         uint8_t* item_status) const;
     Status recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
                                               uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const;
+    Status recover_blobs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells, uint8_t* out_blobs,
+                               uint8_t* item_status) const;
     Status verify_blob_cell_proofs_batch(uint64_t n, const uint8_t* blobs, const uint8_t* commitments, const uint8_t* proofs,
                                          uint8_t* item_status, uint8_t* cell_status, bool* all_ok) const;
 

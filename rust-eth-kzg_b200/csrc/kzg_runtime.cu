@@ -1,5 +1,6 @@
 // Host runtime of the B200 KZG backend (see kzg_runtime.h).
 #include "kzg_runtime.h"
+#include <algorithm>
 #include <cstdio>
 #include <cstdlib>
 #include <ctime>
@@ -144,10 +145,12 @@ Status Workspace::ensure_recover_buffers() {
         EKZG_CUDA(cudaMallocHost(&h_slotmap, (size_t)capacity * 128 * sizeof(int16_t)));
         EKZG_CUDA(cudaMalloc(&d_ze, (size_t)capacity * 128 * sizeof(Fr)));
         EKZG_CUDA(cudaMalloc(&d_czinv, (size_t)capacity * 128 * sizeof(Fr)));
+        EKZG_CUDA(cudaMalloc(&d_cell_off, (size_t)capacity * sizeof(uint32_t)));
+        EKZG_CUDA(cudaMallocHost(&h_cell_off, (size_t)capacity * sizeof(uint32_t)));
         return Status::Ok();
     };
     Status s = all();
-    if (!s.ok) {   // all six or none: a half-built set must never be seen by the next borrower of this workspace
+    if (!s.ok) {   // all or none: a half-built set must never be seen by the next borrower of this workspace
         free_recover_buffers();
         cudaGetLastError();
         return s;
@@ -158,7 +161,9 @@ Status Workspace::ensure_recover_buffers() {
 
 void Workspace::free_recover_buffers() {
     cudaFree(d_rcells); cudaFreeHost(h_rcells); cudaFree(d_slotmap); cudaFreeHost(h_slotmap); cudaFree(d_ze); cudaFree(d_czinv);
+    cudaFree(d_cell_off); cudaFreeHost(h_cell_off);
     d_rcells = nullptr; h_rcells = nullptr; d_slotmap = nullptr; h_slotmap = nullptr; d_ze = nullptr; d_czinv = nullptr;
+    d_cell_off = nullptr; h_cell_off = nullptr;
 }
 
 Status Workspace::ensure_verify_buffers(int blobs) {
@@ -993,19 +998,9 @@ static int rev7(int x) {
     return r;
 }
 
-Status Context::recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
-                                                   uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const {
-    return recover_impl(n, counts, indices, cells, out_cells, out_proofs, item_status, false);
-}
-
-Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells, uint8_t* out_cells,
-                             uint8_t* out_proofs, uint8_t* item_status, bool strided) const {
-    if (n == 0) return Status::Ok();
-    EKZG_TRY(bind_device());
-    // host-side validation in the reference's order (recovery.rs:90-146); invalid items are skipped on the device
-    std::vector<uint64_t> offset(n + 1, 0);
-    for (uint64_t i = 0; i < n; i++) offset[i + 1] = strided ? (i + 1) * (uint64_t)N_CELLS : offset[i] + counts[i];
-    std::vector<uint8_t> code(n, 0);
+// Host-side validation of n recovery items in the reference's order (recovery.rs:90-146): item i has counts[i] indices at
+// indices + offset[i].  Marks every invalid item ITEM_BAD_INDICES in code[] and returns the error of the first one ("" if none).
+static std::string check_recovery_indices(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint64_t* offset, uint8_t* code) {
     std::string first_err;
     for (uint64_t i = 0; i < n; i++) {
         const uint64_t* idx = indices + offset[i];
@@ -1022,6 +1017,37 @@ Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t*
             if (first_err.empty()) first_err = err;
         }
     }
+    return first_err;
+}
+
+// The slot map of one item: sm[m] = rank of the given cell at bit-reversed domain position m, or -1.  An invalid item gets a
+// harmless well-formed instance instead: all cells present (the caller points the device at 128 zero cells for it).
+static void fill_slotmap(int16_t* sm, const uint64_t* idx, uint64_t count, bool invalid) {
+    if (invalid) {
+        for (int m = 0; m < N_CELLS; m++) sm[m] = (int16_t)m;
+        return;
+    }
+    for (int m = 0; m < N_CELLS; m++) sm[m] = -1;
+    for (uint64_t k = 0; k < count; k++) sm[rev7((int)idx[k])] = (int16_t)k;
+}
+
+// ItemStatus of a valid item from the status bits of the recovery kernels (nonzero)
+static uint8_t recovery_device_code(uint32_t bits) { return (bits & 1) ? ITEM_NON_CANONICAL : ITEM_BAD_DEGREE; }
+
+Status Context::recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
+                                                   uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const {
+    return recover_impl(n, counts, indices, cells, out_cells, out_proofs, item_status, false);
+}
+
+Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells, uint8_t* out_cells,
+                             uint8_t* out_proofs, uint8_t* item_status, bool strided) const {
+    if (n == 0) return Status::Ok();
+    EKZG_TRY(bind_device());
+    // host-side validation in the reference's order (recovery.rs:90-146); invalid items are skipped on the device
+    std::vector<uint64_t> offset(n + 1, 0);
+    for (uint64_t i = 0; i < n; i++) offset[i + 1] = strided ? (i + 1) * (uint64_t)N_CELLS : offset[i] + counts[i];
+    std::vector<uint8_t> code(n, 0);
+    std::string first_err = check_recovery_indices(n, counts, indices, offset.data(), code.data());
     const int cap = (int)std::min<uint64_t>(n, (uint64_t)chunk_capacity());
     Workspace* wsp = acquire(proof_route(n, cap, true).capacity, true);
     if (!wsp) return Status::Error("device/pinned memory allocation failed");
@@ -1038,13 +1064,11 @@ Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t*
             int16_t* sm = ws.h_slotmap + (size_t)i * 128;
             const uint64_t g = first + i;
             uint8_t* d_row = ws.d_rcells + (size_t)i * N_CELLS * BYTES_PER_CELL;
-            if (code[g]) {  // give the device a harmless well-formed instance: all cells present, all zero
-                for (int m = 0; m < 128; m++) sm[m] = (int16_t)m;
+            fill_slotmap(sm, indices + offset[g], counts[g], code[g] != 0);
+            if (code[g]) {  // the harmless instance's cells: all zero
                 EKZG_CUDA(cudaMemsetAsync(d_row, 0, (size_t)N_CELLS * BYTES_PER_CELL, st));
                 continue;
             }
-            for (int m = 0; m < 128; m++) sm[m] = -1;
-            for (uint64_t k = 0; k < counts[g]; k++) sm[rev7((int)indices[offset[g] + k])] = (int16_t)k;
             const uint8_t* src = cells + offset[g] * BYTES_PER_CELL;
             const size_t bytes = (size_t)counts[g] * BYTES_PER_CELL;
             if (!in_pinned) {
@@ -1079,7 +1103,7 @@ Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t*
         for (int i = 0; i < cnt; i++) {
             const uint64_t g = first + i;
             if (!code[g] && ws.h_status[i]) {
-                code[g] = (ws.h_status[i] & 1) ? ITEM_NON_CANONICAL : ITEM_BAD_DEGREE;
+                code[g] = recovery_device_code(ws.h_status[i]);
                 if (first_err.empty()) first_err = item_status_text(code[g], true, false);
             }
         }
@@ -1089,6 +1113,132 @@ Status Context::recover_impl(uint64_t n, const uint64_t* counts, const uint64_t*
     give_back(wsp, result);
     if (item_status) memcpy(item_status, code.data(), n);
     if (!result.ok) return result;
+    if (!first_err.empty()) return Status::Error(first_err);
+    return Status::Ok();
+}
+
+// Blobs from their cells, without proofs: R0..R3 of the recovery, then only the first half of the extension (the blob).  With no
+// FK20 behind them the kernels take about as long as the copies (up to 256 KiB of cells up, 128 KiB of blob down per item), so
+// this path is a pipeline: chunks alternate over two workspaces as in compute_cells_and_kzg_proofs_batch, and a chunk is cut
+// into pieces whose cells go up on in_stream, run through the kernels on `stream` and whose blobs go home on copy_stream, each
+// piece a step behind the one before.  The cells go up as the caller packed them (k_recover_ntt_packed reads them through a
+// per-blob offset table): one copy per run of valid items, with no re-layout on the host.
+Status Context::recover_blobs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells, uint8_t* out_blobs,
+                                    uint8_t* item_status) const {
+    if (n == 0) return Status::Ok();
+    EKZG_TRY(bind_device());
+    std::vector<uint64_t> offset(n + 1, 0);
+    for (uint64_t i = 0; i < n; i++) offset[i + 1] = offset[i] + counts[i];
+    std::vector<uint8_t> code(n, 0);
+    std::string first_err = check_recovery_indices(n, counts, indices, offset.data(), code.data());
+    const int cap = (int)std::min<uint64_t>(n, (uint64_t)chunk_capacity());
+    const uint64_t nchunks = (n + cap - 1) / cap;
+    Workspace* W[2] = {acquire(cap, true), nchunks > 1 ? acquire(cap, true) : nullptr};
+    Status result = Status::Ok();
+    if (!W[0] || (nchunks > 1 && !W[1])) result = Status::Error("device/pinned memory allocation failed");
+    for (Workspace* w : W)
+        if (w && result.ok) result = w->ensure_recover_buffers();
+    if (!result.ok) {
+        for (Workspace* w : W) if (w) give_back(w, result);
+        return result;
+    }
+    const bool in_pinned = host_range_is_pinned(cells), out_pinned = host_range_is_pinned(out_blobs);
+    TraceClock tr("recover_blobs_batch");
+    uint64_t pending_first[2] = {0, 0};
+    int pending_cnt[2] = {0, 0}, pending_np[2] = {0, 0};
+    int piece_off[2][Workspace::MAX_SUB], piece_len[2][Workspace::MAX_SUB];
+    auto drain = [&](int slot) -> Status {
+        Workspace& ws = *W[slot];
+        if (!pending_cnt[slot]) return Status::Ok();
+        const uint64_t first = pending_first[slot];
+        for (int s = 0; s < pending_np[slot]; s++) {
+            EKZG_CUDA(cudaEventSynchronize(ws.sub_out[s]));
+            const int o = piece_off[slot][s], c = piece_len[slot][s];
+            if (!out_pinned) memcpy(out_blobs + (first + o) * BYTES_PER_BLOB, ws.h_blobs + (size_t)o * BYTES_PER_BLOB, (size_t)c * BYTES_PER_BLOB);
+        }
+        EKZG_CUDA(cudaEventSynchronize(ws.done));
+        for (int i = 0; i < pending_cnt[slot]; i++)
+            if (!code[first + i] && ws.h_status[i]) code[first + i] = recovery_device_code(ws.h_status[i]);
+        pending_cnt[slot] = 0;
+        return Status::Ok();
+    };
+    auto submit = [&](int slot, uint64_t first, int cnt) -> Status {
+        Workspace& ws = *W[slot];
+        const cudaStream_t st = ws.stream;
+        int np = 0;
+        int* off = piece_off[slot];
+        int* len = piece_len[slot];
+        const int n_p = std::min(Workspace::MAX_SUB, (cnt + 127) / 128), per = (cnt + n_p - 1) / n_p;
+        for (int o = 0; o < cnt; o += per) { off[np] = o; len[np++] = std::min(per, cnt - o); }
+        EKZG_CUDA(cudaStreamWaitEvent(ws.in_stream, ws.done, 0));   // (the previous chunk of this workspace has left the buffers)
+        EKZG_CUDA(cudaMemsetAsync(ws.d_status, 0, sizeof(uint32_t) * cnt, st));
+        // Valid items' cells are packed from cell 0 of d_rcells on; they fill at most 128 (cnt - invalid items) cells, so with an
+        // invalid item in the chunk the last 128 cells of the chunk's rows are free: zeroed, they are the cells of every invalid item.
+        const uint64_t zero_off = (uint64_t)(cnt - 1) * N_CELLS;
+        if (std::any_of(code.begin() + first, code.begin() + first + cnt, [](uint8_t c) { return c != 0; }))
+            EKZG_CUDA(cudaMemsetAsync(ws.d_rcells + zero_off * BYTES_PER_CELL, 0, (size_t)N_CELLS * BYTES_PER_CELL, ws.in_stream));
+        uint64_t packed = 0;   // cells of the chunk's valid items so far
+        for (int s = 0; s < np; s++) {
+            const int o = off[s], c = len[s];
+            for (int i = o; i < o + c;) {
+                const uint64_t g = first + i;
+                if (code[g]) {
+                    fill_slotmap(ws.h_slotmap + (size_t)i * N_CELLS, nullptr, 0, true);
+                    ws.h_cell_off[i++] = (uint32_t)zero_off;
+                    continue;
+                }
+                int j = i;   // a run of valid items [i, j): their cells are contiguous in the caller's buffer and on the device
+                for (; j < o + c && !code[first + j]; j++) {
+                    fill_slotmap(ws.h_slotmap + (size_t)j * N_CELLS, indices + offset[first + j], counts[first + j], false);
+                    ws.h_cell_off[j] = (uint32_t)(packed + offset[first + j] - offset[g]);
+                }
+                const uint64_t run = offset[first + j] - offset[g];
+                EKZG_TRY(upload(ws.d_rcells + packed * BYTES_PER_CELL, ws.h_rcells + packed * BYTES_PER_CELL, cells + offset[g] * BYTES_PER_CELL,
+                                BYTES_PER_CELL, 0, (int)run, in_pinned, ws.in_stream));
+                packed += run;
+                i = j;
+            }
+            EKZG_CUDA(cudaMemcpyAsync(ws.d_slotmap + (size_t)o * N_CELLS, ws.h_slotmap + (size_t)o * N_CELLS, (size_t)c * N_CELLS * sizeof(int16_t),
+                                      cudaMemcpyHostToDevice, ws.in_stream));
+            EKZG_CUDA(cudaMemcpyAsync(ws.d_cell_off + o, ws.h_cell_off + o, (size_t)c * sizeof(uint32_t), cudaMemcpyHostToDevice, ws.in_stream));
+            EKZG_CUDA(cudaEventRecord(ws.piece_in[s], ws.in_stream));
+            EKZG_CUDA(cudaStreamWaitEvent(st, ws.piece_in[s], 0));
+            EKZG_CUDA(launch_recover_coeffs(ws.d_rcells, ws.d_slotmap + (size_t)o * N_CELLS, ws.d_ze + (size_t)o * N_CELLS, ws.d_czinv + (size_t)o * N_CELLS,
+                                            reinterpret_cast<Fr*>(ws.d_scalars) + (size_t)o * N_EXT, reinterpret_cast<Fr*>(ws.d_cells) + (size_t)o * N_EXT,
+                                            ws.d_coeffs + (size_t)o * N_BLOB, ws.d_status + o, T_, coset_shift_fwd_, coset_shift_inv_,
+                                            fr_coset_gen_pow64().v, c, st, ws.d_cell_off + o));
+            EKZG_CUDA(launch_coeffs_to_blob(ws.d_coeffs + (size_t)o * N_BLOB, ws.d_blobs + (size_t)o * BYTES_PER_BLOB, T_, c, st));
+            EKZG_CUDA(cudaEventRecord(ws.sub_ready[s], st));
+            EKZG_CUDA(cudaStreamWaitEvent(ws.copy_stream, ws.sub_ready[s], 0));
+            uint8_t* dst = out_pinned ? out_blobs + (first + o) * BYTES_PER_BLOB : ws.h_blobs + (size_t)o * BYTES_PER_BLOB;
+            EKZG_CUDA(cudaMemcpyAsync(dst, ws.d_blobs + (size_t)o * BYTES_PER_BLOB, (size_t)c * BYTES_PER_BLOB, cudaMemcpyDeviceToHost, ws.copy_stream));
+            EKZG_CUDA(cudaEventRecord(ws.sub_out[s], ws.copy_stream));
+        }
+        EKZG_CUDA(cudaMemcpyAsync(ws.h_status, ws.d_status, sizeof(uint32_t) * cnt, cudaMemcpyDeviceToHost, st));
+        EKZG_CUDA(cudaStreamWaitEvent(st, ws.sub_out[np - 1], 0));   // `done` also covers the last blobs' D2H
+        EKZG_CUDA(cudaEventRecord(ws.done, st));
+        pending_first[slot] = first;
+        pending_cnt[slot] = cnt;
+        pending_np[slot] = np;
+        tr.mark("chunk enqueued");
+        return Status::Ok();
+    };
+    for (uint64_t c = 0; c < nchunks && result.ok; c++) {
+        const int slot = (int)(c & 1);
+        result = drain(slot);
+        if (result.ok) result = submit(slot, c * cap, (int)std::min<uint64_t>(cap, n - c * cap));
+    }
+    for (int slot = 0; slot < 2; slot++) {
+        if (!W[slot]) continue;
+        if (result.ok) result = drain(slot);
+        give_back(W[slot], result);
+    }
+    tr.mark("H2D + kernels + D2H of the chunks");
+    if (item_status) memcpy(item_status, code.data(), n);
+    if (!result.ok) return result;
+    if (first_err.empty())   // no index errors: the first item the device flagged, as recover_impl reports it
+        for (uint64_t i = 0; i < n && first_err.empty(); i++)
+            if (code[i]) first_err = item_status_text(code[i], true, false);
     if (!first_err.empty()) return Status::Error(first_err);
     return Status::Ok();
 }

@@ -97,7 +97,9 @@ struct Workspace {
     int16_t* h_slotmap = nullptr;
     Fr* d_ze = nullptr;            // [cap][128]
     Fr* d_czinv = nullptr;
-    bool recover_ready = false;    // all six recovery buffers exist
+    uint32_t* d_cell_off = nullptr;   // [cap] recover_blobs_batch: first cell of blob i in the packed d_rcells
+    uint32_t* h_cell_off = nullptr;
+    bool recover_ready = false;    // all eight recovery buffers exist
     Status ensure_recover_buffers();
     void free_recover_buffers();
     // verify_blob_cell_proofs_batch (allocated on first use, for the blobs per chunk a call needs -- not the workspace capacity,
@@ -176,6 +178,10 @@ public:
     // out_* contiguous per blob (128*2048 B, 128*48 B).
     Status recover_cells_and_kzg_proofs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells,
                                               uint8_t* out_cells, uint8_t* out_proofs, uint8_t* item_status) const;
+    // The same recovery without proofs: out_blobs n x 131072 B, cells 0..63 of what the call above returns for the valid items.
+    // Inputs, validation order, item_status and error texts as there; the blobs of invalid items are unspecified.
+    Status recover_blobs_batch(uint64_t n, const uint64_t* counts, const uint64_t* indices, const uint8_t* cells, uint8_t* out_blobs,
+                               uint8_t* item_status) const;
 
     // Verifiers.  Err = malformed input, Ok + *verified = false = the proof does not check (bindings/c/src/lib.rs:272-280).
     Status verify_cell_kzg_proof_batch(uint64_t n_commitments, const uint8_t* const* commitments, uint64_t n_indices,

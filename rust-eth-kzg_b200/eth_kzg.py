@@ -70,7 +70,7 @@ def load_library():
                  "eth_kzg_b200_das_context_new_from_json", "eth_kzg_b200_debug_parse_trusted_setup_json", "eth_kzg_b200_debug_g2_keys"):
         getattr(lib, name).restype = _CResult
     for name in ("eth_kzg_b200_verify_cell_kzg_proof_batch_groups", "eth_kzg_b200_verify_blob_kzg_proof_batch_items",
-                 "eth_kzg_b200_verify_blob_cell_proofs_batch"):
+                 "eth_kzg_b200_verify_blob_cell_proofs_batch", "eth_kzg_b200_recover_blobs_batch", "eth_kzg_b200_recover_blob"):
         if hasattr(lib, name):   # (an EKZG_LIB build from before these entry points lacks them)
             getattr(lib, name).restype = _CResult
     _lib = lib
@@ -208,6 +208,18 @@ class DASContext:
                                                                      C.c_uint64(len(cell_indices)), idx, oc, op))
         del keep
         return [b.raw for b in cb], [b.raw for b in pb]
+
+    def recover_blob(self, cell_indices, cells):
+        """the blob (cells 0..63) from at least 64 of its 128 cells, without computing cell proofs.  Raises KzgError exactly
+        where recover_cells_and_kzg_proofs does, with the same message."""
+        cells = [_exact(c, BYTES_PER_CELL, "cell") for c in cells]
+        arr, keep = _ptr_array(cells)
+        idx = (C.c_uint64 * max(len(cell_indices), 1))(*cell_indices)
+        out = C.create_string_buffer(BYTES_PER_BLOB)
+        _check(self._lib, self._lib.eth_kzg_b200_recover_blob(C.c_void_p(self._ctx), C.c_uint64(len(cells)), arr,
+                                                              C.c_uint64(len(cell_indices)), idx, out))
+        del keep
+        return out.raw
 
     # ---- EIP-7594 verifier (crates/eip7594/src/verifier.rs:72) --------------------------------
     def verify_cell_kzg_proof_batch(self, commitments, cell_indices, cells, proofs):
@@ -364,6 +376,20 @@ class DASContext:
         res = self._lib.eth_kzg_b200_recover_cells_and_kzg_proofs_batch(C.c_void_p(self._ctx), C.c_uint64(n), counts, idx, cells, oc, op, status)
         st = _batch_status(self._lib, res, status, n)
         return oc.raw, op.raw, st
+
+    def recover_blobs_batch(self, indices_per_blob, cells_per_blob):
+        """recover_cells_and_kzg_proofs_batch without proofs -> (blobs_flat (n*131072 B), status); the blobs of items with a
+        nonzero status are unspecified"""
+        n = len(indices_per_blob)
+        counts = (C.c_uint64 * max(n, 1))(*[len(x) for x in indices_per_blob])
+        flat_idx = [i for x in indices_per_blob for i in x]
+        idx = (C.c_uint64 * max(len(flat_idx), 1))(*flat_idx)
+        cells = b"".join(_exact(c, BYTES_PER_CELL, "cell") for x in cells_per_blob for c in x)
+        out = C.create_string_buffer(max(n, 1) * BYTES_PER_BLOB)
+        status = C.create_string_buffer(max(n, 1))
+        res = self._lib.eth_kzg_b200_recover_blobs_batch(C.c_void_p(self._ctx), C.c_uint64(n), counts, idx, cells, out, status)
+        st = _batch_status(self._lib, res, status, n)
+        return out.raw[:n * BYTES_PER_BLOB], st
 
     def compute_cells_and_kzg_proofs_device(self, n, d_blobs, d_cells, d_proofs, d_status, stream=0):
         """device pointers (ints), asynchronous on `stream`"""

@@ -9,7 +9,8 @@ Calls: compute_cells_and_kzg_proofs batch (1, 2, 8, 33, 1024 blobs), the device 
 (1, 40), blob_to_kzg_commitment batch and compute_blob_kzg_proof batch (1, 40), compute_kzg_proof (1 call, 40 calls), the
 verifiers verify_cell_kzg_proof_batch (128 and 16 384 openings) and verify_blob_kzg_proof_batch (1, 20 blobs), and, where the
 build has them, the grouped cell verifier and the per-blob verifier on the same inputs (honest, and with one bad item), and
-verify_blob_cell_proofs_batch on 20 blobs (honest, and with one bad proof).
+verify_blob_cell_proofs_batch on 20 blobs (honest, and with one bad proof), and recover_blobs_batch (1, 40) on the recovery
+batch's inputs.
 Each call runs once before it is counted, so first-use allocations are not part of it."""
 import argparse
 import ctypes as C
@@ -126,6 +127,10 @@ def main():
         for name, p in (("honest", cp), ("one_bad", cp_bad)):
             res["verify_blob_cell_proofs_20_%s" % name] = record(
                 lib, lambda p=p: ctx.verify_blob_cell_proofs_batch(flat[:20 * 131072], cms[:20 * 48], p, 20, want_cells=True))
+    if hasattr(lib, "eth_kzg_b200_recover_blobs_batch"):
+        rcl = [[cells[(b * 128 + j) * 2048:(b * 128 + j + 1) * 2048] for j in idx[b]] for b in range(40)]   # (`cl` was reused above)
+        for n in (1, 40):
+            res["recover_blobs_batch_%d" % n] = record(lib, lambda n=n: ctx.recover_blobs_batch(idx[:n], rcl[:n]))
     ctx.close()
 
     with open(args.out, "w") as f:
